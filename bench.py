@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the FruitNeRF per-ray rendering hot path (BASELINE.json metric), one JSON line on stdout.
 
-  python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision fp32|mixed]
+  python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision fp32|mixed] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline `value`: training rays/s (fwd + bwd + gradient all-reduce + Adam) of the `fruit_nerf` preset
@@ -185,6 +185,25 @@ def bytes_of(batch):
     return int(sum(v.numel() * v.element_size() for v in batch.values()))
 
 
+DUMP_PARAM_FLOATS = 15 << 20   # --dump-outputs: parameter values written, all groups together (60 MiB of float32)
+
+
+def last_step_outputs(trainer, stats):
+    """What the caller of the last timed training step is left with: the loss / metric scalars the step returns and the parameters it
+    updated.  A flat group larger than its share of DUMP_PARAM_FLOATS is written as a fixed sample (seeded, sorted indices), so that two
+    builds of the project run with the same arguments write the same elements."""
+    out = {k: v.detach().float().cpu().numpy() for k, v in stats.items()}
+    share = DUMP_PARAM_FLOATS // len(trainer.groups)
+    for name, g in trainer.groups.items():
+        n = g.flat.numel()
+        if n <= share:
+            out["params_" + name] = g.flat.cpu().numpy()
+        else:
+            idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:share].sort().values
+            out[f"params_{name}_sample"] = g.flat[idx.to(g.flat.device)].cpu().numpy()
+    return out
+
+
 def measure(args, precision, dev, world, rank, local_rank, full=True):
     """One precision mode: training step (resident + end-to-end), per-stage device times, eval render."""
     from cropnerf_b200 import _lib as L
@@ -236,13 +255,15 @@ def measure(args, precision, dev, world, rank, local_rank, full=True):
     b0.record()
     h0 = time.perf_counter()
     for i in range(steps):
-        train_step(step, *resident[step % nb]); step += 1
+        stats = train_step(step, *resident[step % nb]); step += 1
     host_enqueue_ms = 1e3 * (time.perf_counter() - h0) / steps   # host time to ENQUEUE one step (no sync inside): must stay below ms_per_step
     settle()
     b1.record()
     barrier()
     clk = clocks.stop() if (rank == 0 and full) else None
     t_local = b0.elapsed_time(b1) / 1e3
+    # taken before the legs below train on: they overwrite the returned loss buffer and move the parameters
+    outputs = last_step_outputs(trainer, stats) if (args.dump_outputs and full and rank == 0) else None
     barrier()  # rank 0 has just spent ~0.2 s stopping its clock sampler: line the ranks up again
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     for i in range(steps):
@@ -463,7 +484,7 @@ def measure(args, precision, dev, world, rank, local_rank, full=True):
         assert not trainer.comm.timed_out(), "a peer-memory barrier timed out during the benchmark"
     del trainer, model, l2_flush
     torch.cuda.empty_cache()
-    return {"ddp": ddp_mode, "host_enqueue_ms": host_enqueue_ms, "ddp_breakdown": ddp_breakdown, "replicas_identical": replicas_identical, "t_dev_batches": t_dev_batches, "t_b2b": t_b2b, "steps": steps, "t": t, "t_e2e": t_e2e, "t_render": t_render, "t_render_e2e": t_render_e2e, "n_r": n_r, "Rr": Rr, "clk": clk,
+    return {"outputs": outputs, "ddp": ddp_mode, "host_enqueue_ms": host_enqueue_ms, "ddp_breakdown": ddp_breakdown, "replicas_identical": replicas_identical, "t_dev_batches": t_dev_batches, "t_b2b": t_b2b, "steps": steps, "t": t, "t_e2e": t_e2e, "t_render": t_render, "t_render_e2e": t_render_e2e, "n_r": n_r, "Rr": Rr, "clk": clk,
             "stage": stage, "n_prof": n_prof, "nonupdate_ms": nonupdate_ms, "camopt_ms": camopt_ms, "adam_ms": adam_ms, "render_stage": render_stage, "loss": loss_host,
             "h2d_train": bytes_of({k: host[0][k] for k in ("origins", "directions", "camera_indices", "image", "fruit_mask")}), "h2d_render": bytes_of({k: rhost[k] for k in ("origins", "directions", "pixel_area", "camera_indices")}),
             "d2h_render": int(d2h_render)}
@@ -509,6 +530,12 @@ def run_product(args):
     assert args.gpus == world, f"--gpus {args.gpus} but WORLD_SIZE={world} (launch N>1 with torch.distributed.run)"
 
     m = measure(args, args.precision, dev, world, rank, local_rank, full=True)
+    if m["outputs"] is not None:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in m["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     other = "fp32" if args.precision == "mixed" else "mixed"
     m2 = measure(args, other, dev, world, rank, local_rank, full=False) if not args.single_precision else None
     R = RAYS_PER_GPU
@@ -782,7 +809,7 @@ def run_reference(args):
     if rank != 0:
         return
     sample = args.cpu_rays
-    res = cpu_baseline(sample_rays=sample, steps=max(1, min(args.steps, 50)), warmup=max(1, min(args.warmup, 3)))
+    res = cpu_baseline(sample_rays=sample, steps=args.steps, warmup=max(1, min(args.warmup, 3)))
     line = {
         "impl": "reference", "metric": "train_rays_per_s", "value": res["value"], "unit": "rays/s", "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": 1e3 * res["seconds_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -816,7 +843,13 @@ def main():
     ap.add_argument("--export-batch", type=int, default=32768, help="--workload export: rays per rendered batch")
     ap.add_argument("--views", type=int, default=300, help="--workload projection: 1080p views")
     ap.add_argument("--super-clusters", type=int, default=2, help="--workload projection: super-clusters (2 sub-cluster boxes each)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (loss / metric scalars) and the "
+                                                          "parameters it updated (a fixed sample of the large groups) as DIR/<name>.npy, float32, under 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "train"):
+        ap.error("--dump-outputs writes the outputs of the CUDA training step: it needs --impl b200 --workload train")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload != "train":

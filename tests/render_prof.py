@@ -1,6 +1,6 @@
 """Profiling aid: a few eval renders of 32768 rays (the export / projection chunk body) in mixed precision."""
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from cropnerf_b200.rays import RayBundle
 dev = torch.device("cuda:0")

@@ -48,6 +48,22 @@ def test_reference_arm_non_zero_ranks_exit_quietly():
     assert out.returncode == 0 and not [l for l in out.stdout.splitlines() if l.startswith("{")]
 
 
+def test_steps_sets_the_number_of_timed_steps():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "51", "--warmup", "0", "--cpu-rays", "16"],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+    assert d["steps"] == 51 and d["cpu_baseline"]["sample"].endswith("mean of 51")
+
+
+def test_bad_arguments_are_refused_before_any_work(tmp_path):
+    dump = tmp_path / "out"
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(dump)], ["--workload", "export", "--dump-outputs", str(dump)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert out.returncode == 2 and "error:" in out.stderr, (extra, out.stderr[-2000:])
+    assert not dump.exists()
+
+
 def test_committed_product_line_has_every_contract_key_and_consistent_arithmetic():
     path = os.path.join(ROOT, "profiles", "r2_bench_1gpu.json")
     if not os.path.exists(path):

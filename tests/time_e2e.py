@@ -1,5 +1,5 @@
-import sys, time, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, time, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from cropnerf_b200 import engine
 dev = torch.device("cuda:0")

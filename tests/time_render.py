@@ -1,5 +1,5 @@
-import sys, torch, time
-sys.path.insert(0, "/root/repo")
+import os, sys, torch, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from cropnerf_b200.rays import RayBundle
 dev = torch.device("cuda:0")
