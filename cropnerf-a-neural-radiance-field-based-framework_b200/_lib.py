@@ -225,6 +225,9 @@ SIGNATURES = {
     "cnb_mlp_hidden_floats": (_I64, [C.POINTER(Mlp)]),
     "cnb_mlp_fwd": (C.c_int, [C.POINTER(Mlp), _P, _I64, _I64, _P, _P, _P]),
     "cnb_mlp_bwd": (C.c_int, [C.POINTER(Mlp), _P, _I64, _P, _P, _P, _I64, _P, _I64, _P]),
+    "cnb_mlp_mixed_scratch_floats": (_I64, [C.POINTER(Mlp), _I64, _I32]),
+    "cnb_mlp_mixed_fwd": (C.c_int, [C.POINTER(Mlp), _P, _I64, _I64, _P, _P, _I32, _P]),
+    "cnb_mlp_mixed_bwd": (C.c_int, [C.POINTER(Mlp), _P, _I64, _P, _P, _I64, _P, _I64, _P, _P]),
     "cnb_density_field_fwd": (C.c_int, [C.POINTER(DensityField), C.POINTER(Samples), _P, _P, _P]),
     "cnb_density_field_bwd": (C.c_int, [C.POINTER(DensityField), C.POINTER(Samples), _P, _P]),
     "cnb_field_ctx_floats": (_I64, [C.POINTER(Field), _I64, _I32]),

@@ -38,6 +38,19 @@ bool cnb_field_mixed_supported(const cnb_field* f);
 int64_t cnb_field_mixed_ctx_floats(int64_t n, int training);
 float* cnb_field_mixed_dx0(float* ctx, int64_t n);  // d(encoded features), LEVEL-MAJOR [16][n][2], written by the mixed backward
 
+// mlp_mixed.cu: the tensor-core operator for MLPs wider than 64, with the kept activations (`hidden`) and the backward's transient scratch
+// (`work`) in separate caller buffers, so that the field can share one work region between its MLPs
+bool cnb_mlp_mixed_supported(const cnb_mlp* m);
+int64_t cnb_mlp_mixed_hidden_floats(const cnb_mlp* m, int64_t n, int training);
+int64_t cnb_mlp_mixed_work_floats(const cnb_mlp* m, int64_t n);
+int cnb_mlp_mixed_fwd_ws(const cnb_mlp* m, const float* x, int64_t x_stride, int64_t n, float* y, float* hidden, int training, cudaStream_t stream);
+int cnb_mlp_mixed_bwd_ws(const cnb_mlp* m, const float* x, int64_t x_stride, const float* hidden, const float* y, const float* dy, int64_t n, float* dx,
+                         int64_t dx_stride, float* work, cudaStream_t stream);
+int cnb_mlp_mixed_launches(const cnb_mlp* m, bool bwd, bool want_dx);
+// field_fp32.cu: the mixed FruitField for architectures outside the fused kernels (the big / huge presets), and its launch counts
+bool cnb_field_mixed_wide_supported(const cnb_field* f);
+int cnb_field_mixed_wide_launches(const cnb_field* f, bool bwd, bool rays);
+
 // hashgrid.cu, library-internal variants reading d(features) level-major [L][n][2]: the fused field backward's accumulator pair of a
 // thread IS one level's two features, and the level-major scatter warps then read one contiguous 256-byte run per request.
 int cnb_hashgrid_bwd_level_major(const cnb_grid* g, const float* positions, const float* d_out, int64_t n, cudaStream_t stream);

@@ -5,6 +5,8 @@
 // :284-302 (forward).  The fp32 path is the 1e-4-parity mode: it chains the exact building blocks
 // (position warp -> cnb_hashgrid -> cnb_mlp(base) -> trunc_exp/SH/embedding glue -> cnb_mlp(sem)+head, cnb_mlp(rgb))
 // through a caller-provided scratch buffer `ctx`, which also keeps the activations the backward needs.
+#include <algorithm>
+
 #include "field_common.cuh"
 
 namespace {
@@ -14,11 +16,14 @@ inline int up4(int v) { return (v + 3) & ~3; }
 struct CtxLayout {
   int64_t pos, sel, x0, hb, bo, hs, s2, semv, rin, hr, rgbv;  // forward (float offsets)
   int64_t d_bo, d_rin, d_s2, d_x0, d_gs;                      // backward scratch
+  int64_t work;                                               // mixed: the MLP operator's backward work space, shared by the three MLPs
   int64_t total;
   int in0, ob, os, ri, rip;
 };
 
-CtxLayout make_layout(const cnb_field* f, int64_t n, bool training) {
+// exact fp32 (mixed = false) or the mixed path for architectures outside the fused kernels (mixed = true): the same chain and layout, with
+// the MLPs' kept activations in the tensor-core operator's fp16 format (inference: one ping-pong region that the three MLPs take in turn)
+CtxLayout make_layout(const cnb_field* f, int64_t n, bool training, bool mixed = false) {
   CtxLayout c;
   c.in0 = f->base.dims[0];
   c.ob = f->base.dims[f->base.num_layers];
@@ -27,18 +32,32 @@ CtxLayout make_layout(const cnb_field* f, int64_t n, bool training) {
   c.rip = up4(c.ri);
   int64_t o = 0;
   auto take = [&](int64_t per) { int64_t r = o; o += per * n; o = (o + 3) & ~(int64_t)3; return r; };
+  auto take_total = [&](int64_t floats) { int64_t r = o; o += floats; o = (o + 3) & ~(int64_t)3; return r; };
+  auto hidden = [&](const cnb_mlp* m) {
+    if (!mixed) return take(training ? cnb_mlp_hidden_floats(m) : 0);
+    return take_total(cnb_mlp_mixed_hidden_floats(m, n, 1));
+  };
   c.pos = take(3); c.sel = take(1); c.x0 = take(c.in0);
-  c.hb = take(training ? cnb_mlp_hidden_floats(&f->base) : 0);
+  if (mixed && !training) {
+    const int64_t h = std::max(cnb_mlp_mixed_hidden_floats(&f->base, n, 0),
+                               std::max(cnb_mlp_mixed_hidden_floats(&f->sem, n, 0), cnb_mlp_mixed_hidden_floats(&f->rgb, n, 0)));
+    c.hb = c.hs = c.hr = take_total(h);
+  } else {
+    c.hb = hidden(&f->base);
+  }
   c.bo = take(c.ob);
-  c.hs = take(training ? cnb_mlp_hidden_floats(&f->sem) : 0);
+  if (training || !mixed) c.hs = hidden(&f->sem);
   c.s2 = take(c.os); c.semv = take(1); c.rin = take(c.rip);
-  c.hr = take(training ? cnb_mlp_hidden_floats(&f->rgb) : 0);
+  if (training || !mixed) c.hr = hidden(&f->rgb);
   c.rgbv = take(3);
   if (training) {
     c.d_bo = take(c.ob); c.d_rin = take(c.rip); c.d_s2 = take(c.os); c.d_x0 = take(c.in0);
-    c.d_gs = take(f->pass_semantic_gradients ? c.ob : 0);
+    c.d_gs = take(f->pass_semantic_gradients && !mixed ? c.ob : 0);
+    c.work = take_total(mixed ? std::max(cnb_mlp_mixed_work_floats(&f->base, n),
+                                         std::max(cnb_mlp_mixed_work_floats(&f->sem, n), cnb_mlp_mixed_work_floats(&f->rgb, n)))
+                              : 0);
   } else {
-    c.d_bo = c.d_rin = c.d_s2 = c.d_x0 = c.d_gs = o;
+    c.d_bo = c.d_rin = c.d_s2 = c.d_x0 = c.d_gs = c.work = o;
   }
   c.total = o;
   return c;
@@ -155,8 +174,26 @@ int cnb_field_check(const cnb_field* f, const cnb_samples* s, bool bwd) {
   return CNB_OK;
 }
 
+bool cnb_field_mixed_wide_supported(const cnb_field* f) {
+  return f && cnb_mlp_mixed_supported(&f->base) && cnb_mlp_mixed_supported(&f->sem) && cnb_mlp_mixed_supported(&f->rgb);
+}
+
+// kernels launched by cnb_field_fwd / cnb_field_bwd(_rays) on the mixed path for the wide architectures (stage timers of pipeline.cu)
+int cnb_field_mixed_wide_launches(const cnb_field* f, bool bwd, bool rays) {
+  if (!bwd) return 4 + cnb_mlp_mixed_launches(&f->base, false, false) + cnb_mlp_mixed_launches(&f->sem, false, false) +
+                   cnb_mlp_mixed_launches(&f->rgb, false, false);
+  return 4 + (rays ? 1 : 0) + cnb_mlp_mixed_launches(&f->rgb, true, true) + cnb_mlp_mixed_launches(&f->sem, true, false) +
+         cnb_mlp_mixed_launches(&f->base, true, true);
+}
+
+namespace {
+// the mixed path of a field that the fused kernels do not cover
+bool mixed_wide(const cnb_field* f) { return f->precision == CNB_PREC_MIXED && !cnb_field_mixed_supported(f) && cnb_field_mixed_wide_supported(f); }
+}  // namespace
+
 extern "C" int64_t cnb_field_ctx_floats(const cnb_field* f, int64_t n, int32_t training) {
   if (!f || n <= 0) return 0;
+  if (mixed_wide(f)) return make_layout(f, n, training != 0, true).total;
   if (f->precision == CNB_PREC_MIXED) return cnb_field_mixed_ctx_floats(n, training);
   return make_layout(f, n, training != 0).total;
 }
@@ -168,9 +205,11 @@ extern "C" int cnb_field_fwd(const cnb_field* f, const cnb_samples* s, float* de
   const int64_t N = s->num_rays * s->samples_per_ray;
   if (N == 0) return CNB_OK;
   CNB_REQUIRE(density != nullptr, "field_fwd: null density output");
-  if (f->precision == CNB_PREC_MIXED) {
+  const bool wide = mixed_wide(f);
+  if (f->precision == CNB_PREC_MIXED && !wide) {
     if (!cnb_field_mixed_supported(f)) {
-      cnb_set_error("field_fwd: mixed precision is compiled for the base fruit_nerf architecture only (L<=16, widths 64, geo 15, app 32)");
+      cnb_set_error("field_fwd: mixed precision is compiled for the base fruit_nerf architecture (L<=16, widths 64, geo 15, app 32) and for "
+                    "MLPs up to 128 wide");
       return CNB_ERR_UNSUPPORTED;
     }
     CNB_REQUIRE(geo == nullptr || f->geo_feat_dim == 15, "field_fwd: the mixed path exports geo as [N,16]");
@@ -178,24 +217,29 @@ extern "C" int cnb_field_fwd(const cnb_field* f, const cnb_samples* s, float* de
     CNB_REQUIRE(!training || (rgb != nullptr && sem != nullptr), "field_fwd: the mixed training forward keeps both heads' activations for the backward");
     return cnb_field_mixed_fwd(f, s, density, geo, rgb, sem, positions_out, ctx, training, stream);
   }
-  CNB_REQUIRE(ctx != nullptr, "field_fwd: fp32 path needs ctx scratch (cnb_field_ctx_floats)");
-  const CtxLayout c = make_layout(f, N, training != 0);
+  CNB_REQUIRE(ctx != nullptr, "field_fwd: this path needs ctx scratch (cnb_field_ctx_floats)");
+  const CtxLayout c = make_layout(f, N, training != 0, wide);
+  // the three MLPs: exact (mlp.cu / mlp_wide.cu) or the tensor-core operator (mlp_mixed.cu)
+  auto mlp_fwd = [&](const cnb_mlp* m, const float* x, int64_t ld, float* y, int64_t hidden) {
+    if (wide) return cnb_mlp_mixed_fwd_ws(m, x, ld, N, y, ctx + hidden, training, stream);
+    return cnb_mlp_fwd(m, x, ld, N, y, training ? ctx + hidden : nullptr, stream);
+  };
   float* pos = ctx + c.pos; float* sel = ctx + c.sel; float* x0 = ctx + c.x0; float* bo = ctx + c.bo;
   k_positions<<<grid1d(N, 256), 256, 0, stream>>>(*s, f->warp, pos, sel, positions_out);
   if ((rc = cnb_check_launch("field positions"))) return rc;
   if ((rc = cnb_hashgrid_fwd(&f->grid, pos, N, x0, nullptr, stream))) return rc;
-  if ((rc = cnb_mlp_fwd(&f->base, x0, c.in0, N, bo, training ? ctx + c.hb : nullptr, stream))) return rc;
+  if ((rc = mlp_fwd(&f->base, x0, c.in0, bo, c.hb))) return rc;
   k_mid_fwd<<<grid1d(N, 256), 256, 0, stream>>>(*s, bo, c.ob, sel, f->embedding, f->mean_embedding, f->appearance_mode, f->appearance_dim, c.rip, density,
                                                  geo, ctx + c.rin);
   if ((rc = cnb_check_launch("field mid"))) return rc;
   if (sem != nullptr || training) {
     float* semv = ctx + c.semv;
-    if ((rc = cnb_mlp_fwd(&f->sem, bo + 1, c.ob, N, ctx + c.s2, training ? ctx + c.hs : nullptr, stream))) return rc;
+    if ((rc = mlp_fwd(&f->sem, bo + 1, c.ob, ctx + c.s2, c.hs))) return rc;
     if ((rc = cnb_mlp_fwd(&f->sem_head, ctx + c.s2, c.os, N, sem ? sem : semv, nullptr, stream))) return rc;
   }
   if (rgb != nullptr || training) {
     float* rgbv = ctx + c.rgbv;
-    if ((rc = cnb_mlp_fwd(&f->rgb, ctx + c.rin, c.rip, N, rgbv, training ? ctx + c.hr : nullptr, stream))) return rc;
+    if ((rc = mlp_fwd(&f->rgb, ctx + c.rin, c.rip, rgbv, c.hr))) return rc;
     if (rgb != nullptr && cudaMemcpyAsync(rgb, rgbv, sizeof(float) * 3 * N, cudaMemcpyDeviceToDevice, stream) != cudaSuccess)
       return cnb_check_launch("field rgb copy");
   }
@@ -208,23 +252,28 @@ extern "C" int cnb_field_bwd(const cnb_field* f, const cnb_samples* s, const flo
   if (rc) return rc;
   const int64_t N = s->num_rays * s->samples_per_ray;
   if (N == 0) return CNB_OK;
+  const bool wide = mixed_wide(f);
   if (f->precision == CNB_PREC_MIXED) {
-    if (!cnb_field_mixed_supported(f)) {
-      cnb_set_error("field_bwd: mixed precision is compiled for the base fruit_nerf architecture only");
+    if (!cnb_field_mixed_supported(f) && !wide) {
+      cnb_set_error("field_bwd: mixed precision is compiled for the base fruit_nerf architecture and for MLPs up to 128 wide");
       return CNB_ERR_UNSUPPORTED;
     }
     CNB_REQUIRE(d_geo == nullptr, "field_bwd: mixed precision path takes no external geo gradient");
     CNB_REQUIRE(ctx != nullptr, "field_bwd: mixed path needs the ctx written by cnb_field_fwd(training=1)");
     CNB_REQUIRE(!f->pass_semantic_gradients, "field_bwd: pass_semantic_gradients is not compiled for the mixed path");
-    return cnb_field_mixed_bwd(f, s, d_density, d_rgb, d_sem, ctx, stream);
+    if (!wide) return cnb_field_mixed_bwd(f, s, d_density, d_rgb, d_sem, ctx, stream);
   }
   CNB_REQUIRE(ctx != nullptr, "field_bwd: fp32 path needs the ctx written by cnb_field_fwd(training=1)");
-  const CtxLayout c = make_layout(f, N, true);
+  const CtxLayout c = make_layout(f, N, true, wide);
+  auto mlp_bwd = [&](const cnb_mlp* m, const float* x, int64_t ld, int64_t hidden, const float* y, const float* dy, float* dx, int64_t dx_ld) {
+    if (wide) return cnb_mlp_mixed_bwd_ws(m, x, ld, ctx + hidden, y, dy, N, dx, dx_ld, ctx + c.work, stream);
+    return cnb_mlp_bwd(m, x, ld, ctx + hidden, y, dy, N, dx, dx_ld, stream);
+  };
   float* pos = ctx + c.pos; float* sel = ctx + c.sel; float* x0 = ctx + c.x0; float* bo = ctx + c.bo;
   float* d_rin = nullptr;
   if (d_rgb != nullptr) {
     d_rin = ctx + c.d_rin;
-    if ((rc = cnb_mlp_bwd(&f->rgb, ctx + c.rin, c.rip, ctx + c.hr, ctx + c.rgbv, d_rgb, N, d_rin, c.rip, stream))) return rc;
+    if ((rc = mlp_bwd(&f->rgb, ctx + c.rin, c.rip, c.hr, ctx + c.rgbv, d_rgb, d_rin, c.rip))) return rc;
     if (f->appearance_mode == CNB_APP_PER_CAMERA && f->d_embedding != nullptr) {
       k_emb_bwd<<<grid1d(s->num_rays, 4), 128, 0, stream>>>(s->camera_indices, s->num_rays, s->samples_per_ray, d_rin, c.rip, 16 + f->geo_feat_dim,
                                                             f->appearance_dim, f->d_embedding);
@@ -238,17 +287,18 @@ extern "C" int cnb_field_bwd(const cnb_field* f, const cnb_samples* s, const flo
       d_gs = ctx + c.d_gs;
       if (cudaMemsetAsync(d_gs, 0, sizeof(float) * c.ob * N, stream) != cudaSuccess) return cnb_check_launch("field memset");
     }
-    if ((rc = cnb_mlp_bwd(&f->sem, bo + 1, c.ob, ctx + c.hs, nullptr, ctx + c.d_s2, N, d_gs ? d_gs + 1 : nullptr, c.ob, stream))) return rc;
+    if ((rc = mlp_bwd(&f->sem, bo + 1, c.ob, c.hs, nullptr, ctx + c.d_s2, d_gs ? d_gs + 1 : nullptr, c.ob))) return rc;
   }
   k_mid_bwd<<<grid1d(N, 256), 256, 0, stream>>>(N, bo, c.ob, sel, d_density, d_rin, c.rip, d_gs, d_geo, ctx + c.d_bo);
   if ((rc = cnb_check_launch("field mid bwd"))) return rc;
-  if ((rc = cnb_mlp_bwd(&f->base, x0, c.in0, ctx + c.hb, nullptr, ctx + c.d_bo, N, ctx + c.d_x0, c.in0, stream))) return rc;
+  if ((rc = mlp_bwd(&f->base, x0, c.in0, c.hb, nullptr, ctx + c.d_bo, ctx + c.d_x0, c.in0))) return rc;
   return cnb_hashgrid_bwd(&f->grid, pos, ctx + c.d_x0, N, stream);
 }
 
 // Same as cnb_field_bwd, plus the gradient with respect to the rays (row a17: camera optimizer): the hash-grid input
 // gradient is chained through the position normalisation / contraction and reduced per ray into d_origins / d_directions
-// (accumulated).  Not compiled for the 16-level limit of the mixed d_x0 layout when num_levels > 16.
+// (accumulated).  Not compiled for the 16-level limit of the fused mixed kernel's d_x0 layout when num_levels > 16; the other paths keep
+// d(features) row-major.
 extern "C" int cnb_field_bwd_rays(const cnb_field* f, const cnb_samples* s, const float* d_density, const float* d_rgb, const float* d_sem,
                                   const float* d_geo, float* ctx, float* d_origins, float* d_directions, cnb_stream_t stream) {
   CNB_REQUIRE(d_origins && d_directions, "field_bwd_rays: null ray gradients");
@@ -256,9 +306,10 @@ extern "C" int cnb_field_bwd_rays(const cnb_field* f, const cnb_samples* s, cons
   if (rc) return rc;
   const int64_t N = s->num_rays * s->samples_per_ray;
   if (N == 0) return CNB_OK;
-  if (f->precision == CNB_PREC_MIXED) {
+  const bool wide = mixed_wide(f);
+  if (f->precision == CNB_PREC_MIXED && !wide) {
     CNB_REQUIRE(f->grid.num_levels == 16, "field_bwd_rays: the mixed path stores d(features) as [16][N][2]; num_levels must be 16");
     return cnb_position_grad_rays_level_major(&f->grid, &f->warp, s, cnb_field_mixed_dx0(ctx, N), d_origins, d_directions, stream);
   }
-  return cnb_position_grad_rays(&f->grid, &f->warp, s, ctx + make_layout(f, N, true).d_x0, d_origins, d_directions, stream);
+  return cnb_position_grad_rays(&f->grid, &f->warp, s, ctx + make_layout(f, N, true, wide).d_x0, d_origins, d_directions, stream);
 }

@@ -34,8 +34,10 @@
 #include <type_traits>
 
 #include "field_mixed.cuh"
+#include "umma.cuh"
 
 using namespace cnbmix;
+using namespace cnbumma;
 
 namespace {
 
@@ -116,31 +118,9 @@ struct BwdArgs {
   long long* dbg;   // CNB_TC5_DEBUG=1: cycle counters of CTA 0 (issuer wait / issue, epilogue wait / work per step)
 };
 
-// ---- tcgen05 plumbing ---------------------------------------------------------------------------------------------------------------------
-// bf16 x bf16 -> f32 ; major: 0 = K, 1 = MN
-__device__ __forceinline__ constexpr uint32_t idesc(int M, int N, int amajor, int bmajor) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)amajor << 15) | ((uint32_t)bmajor << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t id, uint32_t accumulate) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d), "l"(da),
-               "l"(db), "r"(id), "r"(accumulate)
-               : "memory");
-}
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.b32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0;
-  while (!done)
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}" : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-}
+// ---- tcgen05 plumbing (descriptors, umma, tm_load: umma.cuh) -----------------------------------------------------------------------------
 // The issuer is ONE thread: what it executes per MMA is on the critical path of every layer.  A descriptor is built once per GEMM; a K step
-// only adds to the 14-bit start-address field of its low word (shared addresses < 256 KB never carry out of it).
-__device__ __forceinline__ uint32_t desc_lo(uint32_t addr, uint32_t lbo) { return ((addr >> 4) & 0x3FFFu) | ((lbo >> 4) << 16); }
-__device__ __forceinline__ constexpr uint32_t desc_hi(uint32_t sbo) { return (sbo >> 4) | (1u << 14); }
-__device__ __forceinline__ uint64_t desc64(uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | lo; }
+// only adds to the start-address field of its low word.
 template <int KS, uint32_t A_STEP, uint32_t B_STEP>
 __device__ __forceinline__ void mm_loop(uint32_t tm, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t id, bool acc0) {
 #pragma unroll
@@ -164,25 +144,6 @@ __device__ __forceinline__ void mm_dw(uint32_t tm, uint32_t a_s, uint32_t b_s, b
   mm_loop<ROWS / 16, 256, 256>(tm, desc_lo(a_s, 128), desc_hi(FB), desc_lo(b_s, 128), desc_hi(FB), idesc(M, N, 1, 1), !first);
 }
 
-template <int NC>
-__device__ __forceinline__ void tm_load(uint32_t taddr, float (&v)[NC]) {
-  static_assert(NC % 16 == 0, "16-column chunks");
-  uint32_t r[NC];
-#pragma unroll
-  for (int c = 0; c < NC; c += 16)
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                 : "=r"(r[c]), "=r"(r[c + 1]), "=r"(r[c + 2]), "=r"(r[c + 3]), "=r"(r[c + 4]), "=r"(r[c + 5]), "=r"(r[c + 6]), "=r"(r[c + 7]), "=r"(r[c + 8]),
-                   "=r"(r[c + 9]), "=r"(r[c + 10]), "=r"(r[c + 11]), "=r"(r[c + 12]), "=r"(r[c + 13]), "=r"(r[c + 14]), "=r"(r[c + 15])
-                 : "r"(taddr + c));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int c = 0; c < NC; ++c) v[c] = __uint_as_float(r[c]);
-}
-
-__device__ __forceinline__ uint32_t pack_bf2(float a, float b) {
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
 // row-owner store of NB 8-feature blocks (bf16) of this thread's sample row
 template <int NB>
 __device__ __forceinline__ void row_store(unsigned char* mat, int r, const uint32_t (&w)[NB * 4]) {

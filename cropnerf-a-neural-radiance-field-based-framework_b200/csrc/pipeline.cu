@@ -7,7 +7,7 @@
 //   nears,fars [R] | per level: spacing edges [R,S_l+1], euclid edges [R,S_l+1], density [R,S_l], weights [R,S_l]
 //   | field rgb [R,S,3], sem [R,S] | per-ray outputs | (training) per-ray output grads, d_weights/d_density per level,
 //   d_rgb, d_sem | field ctx (cnb_field_ctx_floats)
-#include "cnb_common.cuh"
+#include "field_common.cuh"
 
 #include <cstdio>
 #include <cstdlib>
@@ -170,6 +170,7 @@ int forward_chain(const cnb_model* m, const cnb_rays* rays, const Layout& L, flo
   const cnb_sampler& sp = m->sampler;
   int rc = CNB_OK;
   const bool mixed = m->field.precision == CNB_PREC_MIXED;
+  const bool mixed_wide = mixed && !cnb_field_mixed_supported(&m->field);   // the layer-by-layer tensor-core path (big / huge presets)
   const float* jit = jitter;
   const int lf = L.levels - 1;
   const bool user = out != nullptr;
@@ -202,7 +203,7 @@ int forward_chain(const cnb_model* m, const cnb_rays* rays, const Layout& L, flo
                                                     (lv + 1 == lf && user) ? out->pdf_inds : nullptr, st));
       if (rc) return rc;
     } else {
-      STAGE("field_fwd", mixed ? 1 : 7, cnb_field_fwd(&m->field, &sm, ws + L.dens[lv], nullptr, ws + L.rgb, ws + L.sem, nullptr,
+      STAGE("field_fwd", mixed_wide ? cnb_field_mixed_wide_launches(&m->field, false, false) : (mixed ? 1 : 7), cnb_field_fwd(&m->field, &sm, ws + L.dens[lv], nullptr, ws + L.rgb, ws + L.sem, nullptr,
                                                         L.ctx_floats > 0 ? ws + L.ctx : nullptr, training ? 1 : 0, st));
       if (rc) return rc;
     }
@@ -248,6 +249,7 @@ extern "C" int cnb_train_step(const cnb_model* m, const cnb_rays* rays, const cn
   if ((rc = make_layout(m, R, true, L))) return rc;
   float* ws = workspace;
   const bool mixed = m->field.precision == CNB_PREC_MIXED;
+  const bool mixed_wide = mixed && !cnb_field_mixed_supported(&m->field);   // the layer-by-layer tensor-core path (big / huge presets)
   CNB_REQUIRE(cfg->phase >= 0 && cfg->phase <= 4, "train_step: phase %d outside 0..4", cfg->phase);
   CNB_REQUIRE(cfg->num_opt_groups >= 0 && cfg->num_opt_groups <= CNB_MAX_OPT_GROUPS, "train_step: num_opt_groups %d outside 0..%d", cfg->num_opt_groups, CNB_MAX_OPT_GROUPS);
   // ---- camera optimizer inside the step (row a17): rays are corrected by cnb_camera_opt_apply before the samplers, the kernels return
@@ -315,9 +317,9 @@ extern "C" int cnb_train_step(const cnb_model* m, const cnb_rays* rays, const cn
                                                             m->field.pass_semantic_gradients, losses_out, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, st));
     if (rc) return rc;
     const cnb_samples sm = make_samples(rays, ws + L.eu[lf], Sf);
-    if (rays_grad) STAGE("field_bwd", mixed ? 3 : 9, cnb_field_bwd_rays(&m->field, &sm, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, nullptr, ws + L.ctx,
+    if (rays_grad) STAGE("field_bwd", mixed_wide ? cnb_field_mixed_wide_launches(&m->field, true, true) : (mixed ? 3 : 9), cnb_field_bwd_rays(&m->field, &sm, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, nullptr, ws + L.ctx,
                                                                         d_origins, d_directions, st));
-    else STAGE("field_bwd", mixed ? 2 : 8, cnb_field_bwd(&m->field, &sm, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, nullptr, ws + L.ctx, st));
+    else STAGE("field_bwd", mixed_wide ? cnb_field_mixed_wide_launches(&m->field, true, false) : (mixed ? 2 : 8), cnb_field_bwd(&m->field, &sm, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, nullptr, ws + L.ctx, st));
     if (rc) return rc;
     return optimise(CNB_CHAIN_FIELD, st);  // the field gradient is complete: its Adam pass overlaps the proposal chain
   };

@@ -133,9 +133,10 @@ else:
         return {"optimizer": RAdamOptimizerConfig(lr=1e-2, eps=1e-15),
                 "scheduler": None if lr_final is None else ExponentialDecaySchedulerConfig(lr_final=lr_final, max_steps=max_steps)}
 
-    # The two larger presets (fruit_nerf_config.py:66-190).  Their FruitField is wider than the tensor-core kernels are compiled for (128-wide
-    # three-layer semantic MLP, geo_feat_dim 30), so they run in exact fp32 (`precision="fp32"`: layers above 64 on csrc/mlp_wide.cu); the
-    # optimizers are the reference's (nerfstudio's RAdam; `engine.BIG_PRESET_OPTIMIZERS` is the same for this package's own Trainer).
+    # The two larger presets (fruit_nerf_config.py:66-190).  Their FruitField is wider than the fused kernels (128-wide three-layer semantic MLP,
+    # geo_feat_dim 30).  Registered in exact fp32 (`precision="fp32"`: layers above 64 on csrc/mlp_wide.cu); `--pipeline.model.precision mixed`
+    # runs them as the reference trains them, on the tensor-core operator csrc/mlp_mixed.cu.  The optimizers are the reference's (nerfstudio's
+    # RAdam; `engine.BIG_PRESET_OPTIMIZERS` is the same for this package's own Trainer).
     fruit_nerf_b200_method_big = MethodSpecification(
         config=TrainerConfig(
             method_name="fruit_nerf_b200_big", steps_per_eval_batch=500, steps_per_save=2000, max_num_iterations=100000, mixed_precision=False,

@@ -144,6 +144,20 @@ int cnb_mlp_fwd(const cnb_mlp* m, const float* x, int64_t x_stride, int64_t n, f
 int cnb_mlp_bwd(const cnb_mlp* m, const float* x, int64_t x_stride, const float* hidden, const float* y, const float* dy,
                 int64_t n, float* dx, int64_t dx_stride, cnb_stream_t stream);
 
+/* ---- a3 in mixed precision for layers up to 128 wide (nerfstudio MLP, fruit_field.py:133-167 at the widths of the fruit_nerf_big /
+ *      fruit_nerf_huge presets): tcgen05 tensor cores, fp16 forward operands, bf16 gradient operands, fp32 accumulation
+ *      (csrc/mlp_mixed.cu).  Every width must be 1..128; other shapes return CNB_ERR_UNSUPPORTED with the shape in cnb_last_error.
+ *      Nothing is allocated inside: `scratch` holds the forward's kept activations (training) and the backward's work space, so the calls
+ *      are graph-capturable and independent across streams when each stream has its own scratch. */
+/* floats of `scratch` for n rows; training = 1: what a forward(training=1) + backward pair needs, 0: a forward alone */
+int64_t cnb_mlp_mixed_scratch_floats(const cnb_mlp* m, int64_t n, int32_t training);
+/* as cnb_mlp_fwd; training = 1 keeps the hidden activations in scratch for cnb_mlp_mixed_bwd */
+int cnb_mlp_mixed_fwd(const cnb_mlp* m, const float* x, int64_t x_stride, int64_t n, float* y, float* scratch, int32_t training,
+                      cnb_stream_t stream);
+/* as cnb_mlp_bwd; scratch = the one the forward(training=1) of the same x / n wrote; dW / db accumulated */
+int cnb_mlp_mixed_bwd(const cnb_mlp* m, const float* x, int64_t x_stride, const float* y, const float* dy, int64_t n, float* dx,
+                      int64_t dx_stride, float* scratch, cnb_stream_t stream);
+
 /* ---- a7: HashMLPDensityField.get_density / density_fn (nerfstudio density_fields.py; built fruit_nerf.py:118-142,
  *      handed to the sampler as density_fns fruit_nerf.py:143-145,549) ----------------------------------------------------------- */
 /* density [R*S]; positions_out (optional) [R*S,3] normalised+masked positions */
