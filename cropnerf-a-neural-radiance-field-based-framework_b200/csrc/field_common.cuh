@@ -29,7 +29,7 @@ __device__ __forceinline__ void cnb_sh16(float dx, float dy, float dz, float (&c
 
 int cnb_field_check(const cnb_field* f, const cnb_samples* s, bool bwd);
 
-// mixed-precision (tensor-core) implementation, field_mixed.cu
+// mixed-precision (tensor-core) implementation: field_mixed.cu, the backward in field_mixed_bwd_tc5.cu
 int cnb_field_mixed_fwd(const cnb_field* f, const cnb_samples* s, float* density, float* geo, float* rgb, float* sem, float* positions_out, float* ctx,
                         int training, cudaStream_t stream);
 int cnb_field_mixed_bwd(const cnb_field* f, const cnb_samples* s, const float* d_density, const float* d_rgb, const float* d_sem, float* ctx,

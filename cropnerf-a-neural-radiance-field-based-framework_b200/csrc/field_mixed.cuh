@@ -65,13 +65,14 @@ __device__ __forceinline__ void ldsm_x2(uint32_t (&r)[2], uint32_t addr) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x2.shared.b16 {%0,%1}, [%2];\n" : "=r"(r[0]), "=r"(r[1]) : "r"(addr));
 }
 
-// acc[NT][4] (+)= A[KT][4] x W^T, W = smem [8*NT rows][STRIDE] 16-bit (fp16 or bf16; MMA = the matching mma.sync wrapper).
+// acc[NT][4] (+)= A[KT][4] x W^T, W = smem fp16 [8*NT rows][STRIDE].
 // B fragments come from ldmatrix: one x4 fetches (k 0-7, k 8-15) of TWO n-tiles -- the thread (g, t) of matrix q receives W[row g][2t, 2t+1],
 // which is exactly the col-major B fragment -- instead of four 32-bit shared loads and their address arithmetic (the MLP kernels are
 // issue / latency bound: 15 % of their instructions were those LDS).  Rows are 16-byte aligned (STRIDE % 8 == 0) and STRIDE = 8 (mod 16)
 // halves spreads the eight 16-byte rows of a matrix over all 32 banks.
-template <int NT, int KT, int STRIDE, typename T, typename MMA>
-__device__ __forceinline__ void layer_ldsm(const T* __restrict__ W, const uint32_t (&A)[KT][4], float (&acc)[NT][4], MMA mma) {
+template <int NT, int KT, int STRIDE>
+__device__ __forceinline__ void layer(const __half* __restrict__ W, const uint32_t (&A)[KT][4], float (&acc)[NT][4], int g, int t) {
+  (void)g; (void)t;
   static_assert(STRIDE % 8 == 0, "ldmatrix rows must be 16-byte aligned");
   const int lane = threadIdx.x & 31;
   const uint32_t base = (uint32_t)__cvta_generic_to_shared(W);
@@ -81,7 +82,7 @@ __device__ __forceinline__ void layer_ldsm(const T* __restrict__ W, const uint32
     for (int kt = 0; kt < KT; ++kt) {
       uint32_t b[2];
       ldsm_x2(b, a0 + 2u * kt * 16);
-      mma(acc[0], A[kt], b[0], b[1]);
+      mma_f16(acc[0], A[kt], b[0], b[1]);
     }
   } else {
     static_assert(NT % 2 == 0, "n-tiles are fetched in pairs");
@@ -92,17 +93,11 @@ __device__ __forceinline__ void layer_ldsm(const T* __restrict__ W, const uint32
       for (int kt = 0; kt < KT; ++kt) {
         uint32_t b[4];
         ldsm_x4(b, a0 + 2u * (np * 16 * STRIDE + kt * 16));
-        mma(acc[2 * np], A[kt], b[0], b[1]);
-        mma(acc[2 * np + 1], A[kt], b[2], b[3]);
+        mma_f16(acc[2 * np], A[kt], b[0], b[1]);
+        mma_f16(acc[2 * np + 1], A[kt], b[2], b[3]);
       }
     }
   }
-}
-
-template <int NT, int KT, int STRIDE>
-__device__ __forceinline__ void layer(const __half* __restrict__ W, const uint32_t (&A)[KT][4], float (&acc)[NT][4], int g, int t) {
-  (void)g; (void)t;
-  layer_ldsm<NT, KT, STRIDE>(W, A, acc, [](float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) { mma_f16(c, a, b0, b1); });
 }
 
 template <int NT>

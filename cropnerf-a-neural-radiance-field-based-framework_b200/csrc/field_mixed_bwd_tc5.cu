@@ -1,12 +1,12 @@
 // FruitField backward entirely on tcgen05 / TMEM (rows a1/a5/a6 of SURVEY.md section 8, the autograd of fruit_field.py:169-302).
 //
-// The mma.sync kernel (field_mixed_bwd.cu) keeps a 16-sample tile per warp and chains 13 layers through register fragments: 225 registers,
-// 8 warps per SM, a dependent HMMA -> F2FP -> HMMA chain with nothing to hide it behind (ncu: tensor pipe 26 %, issue 31 %, 30 k cycles per
-// 128-sample batch).  Here a batch of 128 samples is ONE tcgen05.mma tile (M = 128): every layer is 1-4 asynchronous MMAs issued by a single
-// thread, the accumulator lives in tensor memory, and the "epilogue" between two layers is row-parallel -- thread r of a 128-thread
-// warpgroup owns sample r: it reads its accumulator row with tcgen05.ld, applies bias / ReLU / the ReLU mask, converts to bf16 and writes the
-// row back to shared memory as the next layer's operand (8 conflict-free 16-byte stores).  No fragment layouts, no shuffles, ~150
-// instructions per thread and layer.  Two warpgroups work on two batches at once, so one batch's MMAs run under the other's epilogue.
+// An mma.sync design that keeps a 16-sample tile per warp and chains the 13 layers through register fragments needs 225 registers, runs 8 warps per SM
+// and leaves a dependent HMMA -> F2FP -> HMMA chain with nothing to hide it behind (measured: tensor pipe 26 %, issue 31 %, 30 k cycles per 128-sample
+// batch; DESIGN.md section 4).  Here a batch of 128 samples is ONE tcgen05.mma tile (M = 128): every layer is 1-4 asynchronous MMAs issued by a single
+// thread, the accumulator lives in tensor memory, and the "epilogue" between two layers is row-parallel -- thread r of a 128-thread warpgroup owns
+// sample r: it reads its accumulator row with tcgen05.ld, applies bias / ReLU / the ReLU mask, converts to bf16 and writes the row back to shared memory
+// as the next layer's operand (8 conflict-free 16-byte stores).  No fragment layouts, no shuffles, ~150 instructions per thread and layer.  Two
+// warpgroups work on two batches at once, so one batch's MMAs run under the other's epilogue.
 //
 // Shared-memory operand format (no-swizzle canonical UMMA layouts, tests/micro/umma_chain_test.cu):
 //   activation / gradient matrices [128 samples][64 features] bf16:  byte(s, f) = (f/8)*2048 + s*16 + (f%8)*2
@@ -44,11 +44,11 @@ namespace {
 constexpr int ROWS = 128;            // samples per batch = UMMA M = threads of one epilogue warpgroup
 constexpr int NWG = 2;               // batches in flight per CTA
 constexpr int EPI = NWG * ROWS;
-// + two more warpgroups: warps 8, 9 = the layer-MMA issuers of the two epilogue warpgroups, warp 10 = the dW issuer, warps 11..15 = scatter
-// warps (FUSED) or idle.  Registers are re-split after launch with setmaxnreg: 4 x 128 at launch = epilogue 200 + 200, the others 56 + 56
-// (the increase blocks until the decreases have released enough: the sum must not exceed what the CTA was launched with).
+// + two more warpgroups: warps 8, 9 = the layer-MMA issuers of the two epilogue warpgroups, warp 10 = the dW issuer, warps 11..15 idle.
+// The idle warps pay for the epilogue's registers: setmaxnreg re-splits the register file after launch, and the sum must not exceed what
+// the CTA was launched with, so 4 x 128 threads at 128 registers is what lets the epilogue warpgroups rise to 200 (200 + 200 + 56 + 56 =
+// 4 x 128; the increase blocks until the decreases have released enough).
 constexpr int KTHREADS = EPI + 256;
-constexpr int NSC = 5;               // scatter warps (FUSED): warp 11 and the fourth warpgroup
 constexpr uint32_t FB = 2048;        // bytes of one 8-feature block of an activation matrix (128 rows x 16 B)
 constexpr int NSTEP = 12;
 
@@ -106,8 +106,6 @@ static_assert(I_END <= CTX_PART_FLOATS && I_END % 4 == 0, "partial image size");
 struct BwdArgs {
   MixArgs m;
   float* part;      // [gridDim.x][CTX_PART_FLOATS] per-CTA gradient images
-  float* d_table;   // FUSED: gradient table of the hash grid
-  const float* pos; // FUSED: sample positions kept by the forward
   const __half* x0;
   const float* stash;
   const uint4* masks;
@@ -294,45 +292,6 @@ __device__ __forceinline__ void issue_dw(int step, uint32_t tmem, uint32_t wg_s,
   }
 }
 
-// FUSED (CNB_FIELD_BWD_FUSED=1, NOT the default): the hash-table scatter of d(encoded features) inside this kernel, on the five warps of the
-// issuer warpgroups that issue nothing.  The idea: the MLP part is a latency chain that barely touches the LSU (its operands go from shared
-// memory straight to the tensor core), the scatter is bound by the SM's red.global issue rate (tests/micro/table_access_bench) and needs
-// neither shared memory nor many registers, and no second kernel can co-reside with a 219 KB CTA.  Epilogue threads count finished rows in
-// a shared counter (red.release); the scatter warps take the 32-row groups in completion order.  Measured on B200 (4096-ray step): field
-// backward stage 0.281 ms fused vs 0.220 ms as two kernels (0.814 ms with ONE scatter warp): a (32 samples, level) item is a ~2.4 k-cycle
-// dependent chain (L2 read of d_x0 -> cell hash -> segmented scan -> reds), so five warps per SM deliver 480 cycles per item where the
-// stand-alone kernel, with 48 warps per SM, reaches the LSU bound of ~330.  More scatter warps do not fit the register file next to two
-// 200-register epilogue warpgroups.
-__device__ __forceinline__ void scatter_batch(const MixArgs& a, float* __restrict__ d_table, const float* __restrict__ pos, const float* __restrict__ d_x0,
-                                              int64_t batch, int sw, int lane, int64_t N) {
-  {
-    const int64_t s = batch * ROWS + sw * 32 + lane;
-    const bool in = s < N;
-    float px = 0.f, py = 0.f, pz = 0.f;
-    if (in) { px = __ldg(pos + 3 * s); py = __ldg(pos + 3 * s + 1); pz = __ldg(pos + 3 * s + 2); }
-#pragma unroll 1
-    for (int l0 = 0; l0 < a.L; l0 += 4) {
-      float2 d[4];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        d[q] = make_float2(0.f, 0.f);
-        if (in && l0 + q < a.L) d[q] = __ldcg(reinterpret_cast<const float2*>(d_x0) + (int64_t)(l0 + q) * N + s);
-      }
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        const int l = l0 + q;
-        if (l < a.L) {  // warp-uniform
-          const bool active = d[q].x != 0.0f || d[q].y != 0.0f;  // zero gradients add nothing (masked samples, App. B-3)
-          CnbCell c = {};
-          if (active) c = cnb_cell(px, py, pz, a.scalings[l]);
-          cnb_scatter_cell(d_table, c, a.mask, (uint32_t)l * a.T, d[q].x, d[q].y, active);
-        }
-      }
-    }
-  }
-}
-
-template <bool FUSED>
 __global__ void __launch_bounds__(KTHREADS, 1) k_field_bwd_tc5(const __grid_constant__ BwdArgs b) {
   extern __shared__ __align__(1024) unsigned char smem[];
   const MixArgs& a = b.m;
@@ -341,7 +300,6 @@ __global__ void __launch_bounds__(KTHREADS, 1) k_field_bwd_tc5(const __grid_cons
   float* Cf = reinterpret_cast<float*>(smem + O_CONST);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + O_BAR);   // ready[NWG], dwready[NWG] (128 arrivals), done[NWG], dwdone[NWG] (tcgen05.commit)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4 * NWG);
-  uint32_t* rows_done = tmem_slot + 2;   // FUSED: [NWG] rows whose d(encoded features) are in global memory
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   long long tmark[2] = {0, 0};
   load_weights_tc5(a, Wb, Cf, b.dbg ? tmark : nullptr);
@@ -350,7 +308,6 @@ __global__ void __launch_bounds__(KTHREADS, 1) k_field_bwd_tc5(const __grid_cons
   const long long t_w = b.dbg ? clock64() : 0;
   if (threadIdx.x == 0) {
     for (int w = 0; w < NWG; ++w) {
-      rows_done[w] = 0u;
       asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bars + w)), "r"(ROWS));
       asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(bars + NWG + w)), "r"(ROWS));
       asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"((uint32_t)__cvta_generic_to_shared(bars + 2 * NWG + w)));
@@ -421,26 +378,6 @@ __global__ void __launch_bounds__(KTHREADS, 1) k_field_bwd_tc5(const __grid_cons
             }
             __syncwarp();
           }
-        }
-      }
-    } else if (FUSED) {
-      // ===== scatter warps: batch j of this CTA belongs to warpgroup j % NWG and is its (j / NWG)-th; its four 32-row groups are dealt
-      // round-robin over the NSC scatter warps =====
-      const int sc = iw - NWG - 1;   // 0 .. NSC-1
-      const uint32_t cnt_s = (uint32_t)__cvta_generic_to_shared(rows_done);
-      for (int64_t j = 0; j < nb_cta; ++j) {
-        bool waited = false;
-        for (int sw = 0; sw < ROWS / 32; ++sw) {
-          if ((int)((j * (ROWS / 32) + sw) % NSC) != sc) continue;
-          if (!waited) {
-            const uint32_t want = (uint32_t)(j / NWG + 1) * ROWS;
-            uint32_t have;
-            do {
-              asm volatile("ld.acquire.cta.shared::cta.u32 %0, [%1];" : "=r"(have) : "r"(cnt_s + 4u * (uint32_t)(j % NWG)) : "memory");
-            } while (have < want);
-            waited = true;
-          }
-          scatter_batch(a, b.d_table, b.pos, b.d_x0, blockIdx.x + j * gridDim.x, sw, lane, N);
         }
       }
     }
@@ -725,8 +662,6 @@ __global__ void __launch_bounds__(KTHREADS, 1) k_field_bwd_tc5(const __grid_cons
           for (int l = 0; l < 16; ++l)
             if (l < a.L) reinterpret_cast<float2*>(b.d_x0)[(int64_t)l * N + i] = make_float2(v[2 * l], v[2 * l + 1]);
         }
-        if (FUSED)   // release at CTA scope: orders this thread's d_x0 stores before the scatter warp's loads
-          asm volatile("red.release.cta.shared::cta.add.u32 [%0], 1;" ::"r"((uint32_t)__cvta_generic_to_shared(rows_done + wg)) : "memory");
         asm volatile("tcgen05.fence::before_thread_sync;");
         if (dbg_on) { b.dbg[48] += clock64() - te; b.dbg[53] = t_fence; b.dbg[54] = t_dbgrmw; }
       }
@@ -831,8 +766,8 @@ __global__ void __launch_bounds__(256) k_tc5_reduce(const __grid_constant__ BwdA
 
 }  // namespace
 
-int cnb_field_mixed_bwd_tc5(const cnb_field* f, const cnb_samples* s, const float* d_density, const float* d_rgb, const float* d_sem, float* ctx,
-                            cudaStream_t stream) {
+int cnb_field_mixed_bwd(const cnb_field* f, const cnb_samples* s, const float* d_density, const float* d_rgb, const float* d_sem, float* ctx,
+                        cudaStream_t stream) {
   BwdArgs b;
   fill_args(f, s, b.m);
   const int64_t N = s->num_rays * s->samples_per_ray;
@@ -857,22 +792,14 @@ int cnb_field_mixed_bwd_tc5(const cnb_field* f, const cnb_samples* s, const floa
   }
   static bool configured = false;
   if (!configured) {
-    if (cudaFuncSetAttribute(k_field_bwd_tc5<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_TC5) != cudaSuccess ||
-        cudaFuncSetAttribute(k_field_bwd_tc5<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_TC5) != cudaSuccess)
+    if (cudaFuncSetAttribute(k_field_bwd_tc5, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_TC5) != cudaSuccess)
       return cnb_check_launch("field_bwd_tc5 attr");
     configured = true;
   }
   const int64_t nbatches = (N + ROWS - 1) / ROWS;
   int64_t blocks = nbatches < (int64_t)cnb_num_sms() ? nbatches : (int64_t)cnb_num_sms();
   if (blocks > CTX_PART_CTAS) blocks = CTX_PART_CTAS;
-  // default: the table scatter as a second kernel (cnb_hashgrid_bwd_level_major); CNB_FIELD_BWD_FUSED=1: inside this one, same arithmetic
-  static const bool want_fused = [] { const char* e = getenv("CNB_FIELD_BWD_FUSED"); return e != nullptr && e[0] == '1'; }();
-  b.d_table = f->grid.d_table;
-  b.pos = ctx + ctx_pos_off(N);
-  bool fused = want_fused && b.d_table != nullptr;
-  for (int i = 0; i < f->grid.num_levels && fused; ++i) fused = f->grid.scalings[i] < 65535.0f;  // cnb_scatter_cell's 16-bit cell keys
-  if (fused) k_field_bwd_tc5<true><<<(int)blocks, KTHREADS, SMEM_TC5, stream>>>(b);
-  else k_field_bwd_tc5<false><<<(int)blocks, KTHREADS, SMEM_TC5, stream>>>(b);
+  k_field_bwd_tc5<<<(int)blocks, KTHREADS, SMEM_TC5, stream>>>(b);
   int rc = cnb_check_launch("field_bwd_tc5");
   if (rc) return rc;
   k_tc5_reduce<<<dim3((I_END + 255) / 256, 4), 256, 0, stream>>>(b, (int)blocks);
@@ -886,6 +813,5 @@ int cnb_field_mixed_bwd_tc5(const cnb_field* f, const cnb_samples* s, const floa
     fprintf(stderr, "[tc5] final epilogue work %lld ; CTA 0: prologue %lld, batch loop end %lld, kernel end %lld cycles\n", h[48], h[49], h[50], h[51]);
     fprintf(stderr, "[tc5] weights: loads issued at %lld, first matrix stored at %lld, all stored at %lld cycles; fence+arrive total %lld; dbg RMW total %lld\n", h[55], h[56], h[52], h[53], h[54]);
   }
-  if (fused) return CNB_OK;
   return cnb_hashgrid_bwd_level_major(&f->grid, ctx + ctx_pos_off(N), b.d_x0, N, stream);
 }

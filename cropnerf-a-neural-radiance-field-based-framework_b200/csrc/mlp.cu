@@ -3,289 +3,7 @@
 // 159-167) and FieldHead (components/field_heads.py:29-40).  This is the exact-fp32 path (1e-4 parity mode);
 // the mixed-precision hot path fuses the same layers on tensor cores in field_mixed.cu.
 //
-// Layout: one CTA = 128 threads = one tile of 128 samples; weights of every layer resident in shared memory
-// ([out][in] like nn.Linear.weight, rows padded to 4 floats); activations in a row-major smem tile with a
-// 68-float row stride so that each thread's float4 row accesses are bank-conflict free (8 lanes x 16 B per
-// phase land on 32 distinct banks) and weight reads are warp-wide broadcasts.
-#include <cstdlib>
-
-#include "cnb_common.cuh"
-
-namespace {
-
-constexpr int TILE = 128;
-constexpr int ROW = 68;
-
-struct MlpArgs {
-  int nl;
-  int dims[CNB_MAX_LAYERS + 1];
-  int inp[CNB_MAX_LAYERS];   // in dim padded to 4
-  int outp[CNB_MAX_LAYERS];  // out dim padded to 4
-  int wo[CNB_MAX_LAYERS];    // smem offset of W_l
-  int bo[CNB_MAX_LAYERS];    // smem offset of b_l
-  int total_w;               // floats of smem weights+biases
-  int act;
-  const float* W[CNB_MAX_LAYERS];
-  const float* b[CNB_MAX_LAYERS];
-  float* dW[CNB_MAX_LAYERS];
-  float* db[CNB_MAX_LAYERS];
-};
-
-inline int up4(int v) { return (v + 3) & ~3; }
-
-int make_args(const cnb_mlp* m, MlpArgs& a) {
-  CNB_REQUIRE(m != nullptr, "mlp: null descriptor");
-  CNB_REQUIRE(m->num_layers >= 1 && m->num_layers <= CNB_MAX_LAYERS, "mlp: num_layers %d outside 1..%d", m->num_layers, CNB_MAX_LAYERS);
-  a.nl = m->num_layers;
-  a.act = m->out_activation;
-  int off = 0;
-  for (int l = 0; l <= a.nl; ++l) {
-    CNB_REQUIRE(m->dims[l] >= 1 && m->dims[l] <= CNB_MAX_WIDTH, "mlp: dims[%d]=%d outside 1..%d", l, m->dims[l], CNB_MAX_WIDTH);
-    a.dims[l] = m->dims[l];
-  }
-  for (int l = 0; l < CNB_MAX_LAYERS; ++l) {
-    if (l < a.nl) {
-      CNB_REQUIRE(m->W[l] && m->b[l], "mlp: null W/b for layer %d", l);
-      a.inp[l] = up4(a.dims[l]);
-      a.outp[l] = up4(a.dims[l + 1]);
-      a.wo[l] = off;
-      off += a.outp[l] * a.inp[l];
-      a.bo[l] = off;
-      off += a.outp[l];
-      a.W[l] = m->W[l]; a.b[l] = m->b[l]; a.dW[l] = m->dW[l]; a.db[l] = m->db[l];
-    } else {
-      a.inp[l] = a.outp[l] = a.wo[l] = a.bo[l] = 0;
-      a.W[l] = a.b[l] = nullptr; a.dW[l] = a.db[l] = nullptr;
-    }
-  }
-  a.total_w = off;
-  return CNB_OK;
-}
-
-__device__ __forceinline__ void load_weights(const MlpArgs& m, float* Ws) {
-  for (int l = 0; l < m.nl; ++l) {
-    const int in = m.dims[l], out = m.dims[l + 1], inp = m.inp[l], outp = m.outp[l];
-    for (int e = threadIdx.x; e < outp * inp; e += TILE) {
-      const int j = e / inp, k = e - j * inp;
-      Ws[m.wo[l] + e] = (j < out && k < in) ? __ldg(m.W[l] + j * in + k) : 0.0f;
-    }
-    for (int j = threadIdx.x; j < outp; j += TILE) Ws[m.bo[l] + j] = j < out ? __ldg(m.b[l] + j) : 0.0f;
-  }
-}
-
-__device__ __forceinline__ int up16_dev(int v) { return (v + 15) & ~15; }
-
-__device__ __forceinline__ float apply_act(float v, int act) {
-  if (act == CNB_ACT_RELU) return fmaxf(v, 0.0f);
-  if (act == CNB_ACT_SIGMOID) return 1.0f / (1.0f + expf(-v));
-  return v;
-}
-
-// y[0..outp) = act(W x + b) for this thread's own row
-__device__ __forceinline__ void dense_row(const float* __restrict__ xin, const float* __restrict__ W, const float* __restrict__ b,
-                                          int inp, int outp, int act, float* __restrict__ yout) {
-  for (int j0 = 0; j0 < outp; j0 += 4) {
-    float4 bb = *reinterpret_cast<const float4*>(b + j0);
-    float a0 = bb.x, a1 = bb.y, a2 = bb.z, a3 = bb.w;
-    const float* w0 = W + (j0 + 0) * inp;
-    const float* w1 = W + (j0 + 1) * inp;
-    const float* w2 = W + (j0 + 2) * inp;
-    const float* w3 = W + (j0 + 3) * inp;
-    for (int k = 0; k < inp; k += 4) {
-      const float4 xv = *reinterpret_cast<const float4*>(xin + k);
-      const float4 p0 = *reinterpret_cast<const float4*>(w0 + k);
-      const float4 p1 = *reinterpret_cast<const float4*>(w1 + k);
-      const float4 p2 = *reinterpret_cast<const float4*>(w2 + k);
-      const float4 p3 = *reinterpret_cast<const float4*>(w3 + k);
-      a0 = fmaf(p0.x, xv.x, a0); a0 = fmaf(p0.y, xv.y, a0); a0 = fmaf(p0.z, xv.z, a0); a0 = fmaf(p0.w, xv.w, a0);
-      a1 = fmaf(p1.x, xv.x, a1); a1 = fmaf(p1.y, xv.y, a1); a1 = fmaf(p1.z, xv.z, a1); a1 = fmaf(p1.w, xv.w, a1);
-      a2 = fmaf(p2.x, xv.x, a2); a2 = fmaf(p2.y, xv.y, a2); a2 = fmaf(p2.z, xv.z, a2); a2 = fmaf(p2.w, xv.w, a2);
-      a3 = fmaf(p3.x, xv.x, a3); a3 = fmaf(p3.y, xv.y, a3); a3 = fmaf(p3.z, xv.z, a3); a3 = fmaf(p3.w, xv.w, a3);
-    }
-    *reinterpret_cast<float4*>(yout + j0) = make_float4(apply_act(a0, act), apply_act(a1, act), apply_act(a2, act), apply_act(a3, act));
-  }
-}
-
-__global__ void __launch_bounds__(TILE) k_mlp_fwd(MlpArgs m, const float* __restrict__ x, int64_t x_stride, int64_t n, float* __restrict__ y,
-                                                  float* __restrict__ hidden) {
-  extern __shared__ float4 smem4[];
-  float* Ws = reinterpret_cast<float*>(smem4);
-  float* tA = Ws + m.total_w;
-  float* tB = tA + TILE * ROW;
-  load_weights(m, Ws);
-  __syncthreads();
-  const int tid = threadIdx.x;
-  const int64_t ntiles = (n + TILE - 1) / TILE;
-  for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-    const int64_t n0 = tile * TILE;
-    const int cnt = (int)min((int64_t)TILE, n - n0);
-    const int in0 = m.dims[0], inp0 = m.inp[0];
-    for (int e = tid; e < TILE * inp0; e += TILE) {
-      const int r = e / inp0, k = e - r * inp0;
-      tA[r * ROW + k] = (r < cnt && k < in0) ? __ldg(x + (n0 + r) * x_stride + k) : 0.0f;
-    }
-    __syncthreads();
-    float* cur = tA;
-    float* nxt = tB;
-    int64_t hoff = 0;
-    for (int l = 0; l < m.nl; ++l) {
-      const bool last = (l == m.nl - 1);
-      dense_row(cur + tid * ROW, Ws + m.wo[l], Ws + m.bo[l], m.inp[l], m.outp[l], last ? m.act : CNB_ACT_RELU, nxt + tid * ROW);
-      if (!last && hidden != nullptr) {
-        __syncthreads();
-        const int w = m.dims[l + 1];
-        float* dst = hidden + hoff + n0 * w;
-        for (int e = tid; e < cnt * w; e += TILE) {
-          const int r = e / w, k = e - r * w;
-          dst[e] = nxt[r * ROW + k];
-        }
-        hoff += n * (int64_t)w;
-      }
-      float* t = cur; cur = nxt; nxt = t;
-    }
-    __syncthreads();
-    const int out = m.dims[m.nl];
-    for (int e = tid; e < cnt * out; e += TILE) {
-      const int r = e / out, k = e - r * out;
-      y[n0 * out + e] = cur[r * ROW + k];
-    }
-    __syncthreads();
-  }
-}
-
-__global__ void __launch_bounds__(TILE) k_mlp_bwd(MlpArgs m, const float* __restrict__ x, int64_t x_stride, const float* __restrict__ hidden,
-                                                  const float* __restrict__ y, const float* __restrict__ dy, int64_t n, float* __restrict__ dx,
-                                                  int64_t dx_stride) {
-  extern __shared__ float4 smem4[];
-  float* Ws = reinterpret_cast<float*>(smem4);
-  float* dWs = Ws + m.total_w;
-  float* tIn = dWs + m.total_w;
-  float* tD = tIn + TILE * ROW;
-  float* tN = tD + TILE * ROW;
-  const int tid = threadIdx.x;
-  load_weights(m, Ws);
-  for (int e = tid; e < m.total_w; e += TILE) dWs[e] = 0.0f;
-  __syncthreads();
-  const int64_t ntiles = (n + TILE - 1) / TILE;
-  for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-    const int64_t n0 = tile * TILE;
-    const int cnt = (int)min((int64_t)TILE, n - n0);
-    {
-      const int out = m.dims[m.nl], outp = m.outp[m.nl - 1];
-      for (int e = tid; e < TILE * outp; e += TILE) {
-        const int r = e / outp, j = e - r * outp;
-        float v = 0.0f;
-        if (r < cnt && j < out) {
-          v = __ldg(dy + (n0 + r) * out + j);
-          if (m.act == CNB_ACT_SIGMOID) { const float yy = __ldg(y + (n0 + r) * out + j); v *= yy * (1.0f - yy); }
-          else if (m.act == CNB_ACT_RELU) { if (!(__ldg(y + (n0 + r) * out + j) > 0.0f)) v = 0.0f; }
-        }
-        tD[r * ROW + j] = v;
-      }
-    }
-    for (int l = m.nl - 1; l >= 0; --l) {
-      const int in = m.dims[l], inp = m.inp[l], outp = m.outp[l];
-      const float* src;
-      int64_t sstride;
-      if (l == 0) { src = x + n0 * x_stride; sstride = x_stride; }
-      else {
-        int64_t hoff = 0;
-        for (int q = 0; q < l - 1; ++q) hoff += n * (int64_t)m.dims[q + 1];
-        src = hidden + hoff + n0 * in; sstride = in;
-      }
-      for (int e = tid; e < TILE * inp; e += TILE) {
-        const int r = e / inp, k = e - r * inp;
-        tIn[r * ROW + k] = (r < cnt && k < in) ? __ldg(src + r * sstride + k) : 0.0f;
-      }
-      __syncthreads();
-      // (a) dW += dOut^T In over the tile, 4x4 register blocks with fixed thread ownership (no atomics in smem)
-      const int kblocks = inp >> 2;
-      const int nblk = (outp >> 2) * kblocks;
-      for (int b = tid; b < nblk; b += TILE) {
-        const int jb = b / kblocks, kb = b - jb * kblocks;
-        float acc[4][4] = {};
-        const float* dp = tD + 4 * jb;
-        const float* xp = tIn + 4 * kb;
-        for (int s = 0; s < cnt; ++s) {
-          const float4 d4 = *reinterpret_cast<const float4*>(dp + s * ROW);
-          const float4 x4 = *reinterpret_cast<const float4*>(xp + s * ROW);
-          const float dd[4] = {d4.x, d4.y, d4.z, d4.w};
-          const float xx[4] = {x4.x, x4.y, x4.z, x4.w};
-#pragma unroll
-          for (int a = 0; a < 4; ++a)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) acc[a][c] = fmaf(dd[a], xx[c], acc[a][c]);
-        }
-        float* dst = dWs + m.wo[l] + (4 * jb) * inp + 4 * kb;
-#pragma unroll
-        for (int a = 0; a < 4; ++a)
-#pragma unroll
-          for (int c = 0; c < 4; ++c) dst[a * inp + c] += acc[a][c];
-      }
-      if (tid < outp) {
-        float sacc = 0.0f;
-        for (int s = 0; s < cnt; ++s) sacc += tD[s * ROW + tid];
-        dWs[m.bo[l] + tid] += sacc;
-      }
-      // (b) dIn = dOut W, masked by the ReLU of the producing layer
-      if (l > 0 || dx != nullptr) {
-        const float* drow = tD + tid * ROW;
-        const float* W = Ws + m.wo[l];
-        for (int k0 = 0; k0 < inp; k0 += 4) {
-          float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-          for (int j = 0; j < outp; j += 4) {
-            const float4 d4 = *reinterpret_cast<const float4*>(drow + j);
-            const float4 w0 = *reinterpret_cast<const float4*>(W + (j + 0) * inp + k0);
-            const float4 w1 = *reinterpret_cast<const float4*>(W + (j + 1) * inp + k0);
-            const float4 w2 = *reinterpret_cast<const float4*>(W + (j + 2) * inp + k0);
-            const float4 w3 = *reinterpret_cast<const float4*>(W + (j + 3) * inp + k0);
-            a0 = fmaf(d4.x, w0.x, a0); a1 = fmaf(d4.x, w0.y, a1); a2 = fmaf(d4.x, w0.z, a2); a3 = fmaf(d4.x, w0.w, a3);
-            a0 = fmaf(d4.y, w1.x, a0); a1 = fmaf(d4.y, w1.y, a1); a2 = fmaf(d4.y, w1.z, a2); a3 = fmaf(d4.y, w1.w, a3);
-            a0 = fmaf(d4.z, w2.x, a0); a1 = fmaf(d4.z, w2.y, a1); a2 = fmaf(d4.z, w2.z, a2); a3 = fmaf(d4.z, w2.w, a3);
-            a0 = fmaf(d4.w, w3.x, a0); a1 = fmaf(d4.w, w3.y, a1); a2 = fmaf(d4.w, w3.z, a2); a3 = fmaf(d4.w, w3.w, a3);
-          }
-          if (l > 0) {
-            const float4 h = *reinterpret_cast<const float4*>(tIn + tid * ROW + k0);
-            if (!(h.x > 0.f)) a0 = 0.f;
-            if (!(h.y > 0.f)) a1 = 0.f;
-            if (!(h.z > 0.f)) a2 = 0.f;
-            if (!(h.w > 0.f)) a3 = 0.f;
-          }
-          *reinterpret_cast<float4*>(tN + tid * ROW + k0) = make_float4(a0, a1, a2, a3);
-        }
-      }
-      __syncthreads();
-      float* t = tD; tD = tN; tN = t;
-    }
-    if (dx != nullptr) {
-      const int in0 = m.dims[0];
-      for (int e = tid; e < cnt * in0; e += TILE) {
-        const int r = e / in0, k = e - r * in0;
-        dx[(n0 + r) * dx_stride + k] = tD[r * ROW + k];
-      }
-    }
-    __syncthreads();
-  }
-  // flush this CTA's partial sums
-  for (int l = 0; l < m.nl; ++l) {
-    const int in = m.dims[l], out = m.dims[l + 1], inp = m.inp[l];
-    if (m.dW[l])
-      for (int e = tid; e < out * in; e += TILE) {
-        const int j = e / in, k = e - j * in;
-        const float v = dWs[m.wo[l] + j * inp + k];
-        if (v != 0.0f) atomicAdd(m.dW[l] + e, v);
-      }
-    if (m.db[l])
-      for (int j = tid; j < out; j += TILE) {
-        const float v = dWs[m.bo[l] + j];
-        if (v != 0.0f) atomicAdd(m.db[l] + j, v);
-      }
-  }
-}
-
-
-// =====================================================================================================================
-// Tensor-core version of the same exact-fp32 operator: 3xTF32.  Every fp32 operand is split into a tf32 "hi" part and a tf32 "lo"
+// The layers run on tensor cores as 3xTF32.  Every fp32 operand is split into a tf32 "hi" part and a tf32 "lo"
 // residual (x = hi + lo up to 2^-22 relative) and each product is accumulated as hi*hi + lo*hi + hi*lo on
 // mma.sync.m16n8k8.tf32 with fp32 accumulators: ~2^-21 relative error per product (the dropped lo*lo term), i.e. fp32-class
 // results -- the tests' 1e-5 / 2e-5 bounds against the oracle are unchanged -- at tensor-core rate instead of FFMA rate.
@@ -297,6 +15,18 @@ __global__ void __launch_bounds__(TILE) k_mlp_bwd(MlpArgs m, const float* __rest
 // feature, k = sample) with its output tiles dealt round-robin to the 8 warps and accumulated in a per-CTA shared-memory copy of the
 // gradients (fixed ownership, no atomics until the flush); the bias gradient is one more n-tile against a column of ones;
 // dIn = dOut W is row-parallel again (warp = 16 rows).
+#include "cnb_common.cuh"
+
+namespace {
+
+__device__ __forceinline__ int up16_dev(int v) { return (v + 15) & ~15; }
+
+__device__ __forceinline__ float apply_act(float v, int act) {
+  if (act == CNB_ACT_RELU) return fmaxf(v, 0.0f);
+  if (act == CNB_ACT_SIGMOID) return 1.0f / (1.0f + expf(-v));
+  return v;
+}
+
 namespace tc {
 
 constexpr int WARPS = 8;
@@ -320,22 +50,30 @@ struct Args {
 inline int up8(int v) { return (v + 7) & ~7; }
 inline int up16(int v) { return (v + 15) & ~15; }
 
-void make(const MlpArgs& m, Args& a) {
-  a.nl = m.nl; a.act = m.act;
+int make_args(const cnb_mlp* m, Args& a) {
+  CNB_REQUIRE(m != nullptr, "mlp: null descriptor");
+  CNB_REQUIRE(m->num_layers >= 1 && m->num_layers <= CNB_MAX_LAYERS, "mlp: num_layers %d outside 1..%d", m->num_layers, CNB_MAX_LAYERS);
+  a.nl = m->num_layers;
+  a.act = m->out_activation;
+  for (int l = 0; l <= a.nl; ++l) {
+    CNB_REQUIRE(m->dims[l] >= 1 && m->dims[l] <= CNB_MAX_WIDTH, "mlp: dims[%d]=%d outside 1..%d", l, m->dims[l], CNB_MAX_WIDTH);
+    a.dims[l] = m->dims[l];
+  }
   int off = 0;
-  for (int l = 0; l <= m.nl; ++l) a.dims[l] = m.dims[l];
   for (int l = 0; l < CNB_MAX_LAYERS; ++l) {
-    if (l < m.nl) {
-      a.in8[l] = up8(m.dims[l]); a.out8[l] = up8(m.dims[l + 1]); a.ws[l] = a.in8[l] + 4;
-      a.wo[l] = off; off += up16(m.dims[l + 1]) * a.ws[l];   // rows padded to 16: the dW contraction uses m16 tiles
-      a.bo[l] = off; off += up16(m.dims[l + 1]);
-      a.W[l] = m.W[l]; a.b[l] = m.b[l]; a.dW[l] = m.dW[l]; a.db[l] = m.db[l];
+    if (l < a.nl) {
+      CNB_REQUIRE(m->W[l] && m->b[l], "mlp: null W/b for layer %d", l);
+      a.in8[l] = up8(a.dims[l]); a.out8[l] = up8(a.dims[l + 1]); a.ws[l] = a.in8[l] + 4;
+      a.wo[l] = off; off += up16(a.dims[l + 1]) * a.ws[l];   // rows padded to 16: the dW contraction uses m16 tiles
+      a.bo[l] = off; off += up16(a.dims[l + 1]);
+      a.W[l] = m->W[l]; a.b[l] = m->b[l]; a.dW[l] = m->dW[l]; a.db[l] = m->db[l];
     } else {
       a.in8[l] = a.out8[l] = a.ws[l] = a.wo[l] = a.bo[l] = 0;
       a.W[l] = a.b[l] = nullptr; a.dW[l] = a.db[l] = nullptr;
     }
   }
   a.total_w = (off + 3) & ~3;
+  return CNB_OK;
 }
 
 // x = hi + lo with hi a tf32 number (10 mantissa bits) rounded to nearest: two integer ops instead of cvt.rna.tf32.f32 (a conversion-unit
@@ -675,12 +413,6 @@ __global__ void __launch_bounds__(THREADS, 1) k_mlp_bwd_tc(const __grid_constant
 
 }  // namespace
 
-// CNB_MLP_SIMT=1 keeps the FFMA kernels (A/B measurements); default = the 3xTF32 tensor-core kernels
-static bool use_tc() {
-  static const bool simt = [] { const char* e = getenv("CNB_MLP_SIMT"); return e != nullptr && e[0] == '1'; }();
-  return !simt;
-}
-
 // mlp_wide.cu: layer-by-layer path for MLPs with a dimension above CNB_MAX_WIDTH
 bool cnb_mlp_is_wide(const cnb_mlp* m);
 int cnb_mlp_wide_fwd(const cnb_mlp* m, const float* x, int64_t x_stride, int64_t n, float* y, float* hidden, cudaStream_t stream);
@@ -705,37 +437,23 @@ extern "C" int cnb_mlp_fwd(const cnb_mlp* m, const float* x, int64_t x_stride, i
     if (n == 0) return CNB_OK;
     return cnb_mlp_is_lin1(m) ? cnb_mlp_lin1_fwd(m, x, x_stride, n, y, stream) : cnb_mlp_wide_fwd(m, x, x_stride, n, y, hidden, stream);
   }
-  MlpArgs a;
-  int rc = make_args(m, a);
+  tc::Args a;
+  int rc = tc::make_args(m, a);
   if (rc) return rc;
   CNB_REQUIRE(n >= 0 && (n == 0 || (x && y)), "mlp_fwd: null x/y");
   CNB_REQUIRE(x_stride >= a.dims[0], "mlp_fwd: x_stride %lld < in dim %d", (long long)x_stride, a.dims[0]);
   if (n == 0) return CNB_OK;
-  if (use_tc()) {
-    tc::Args ta;
-    tc::make(a, ta);
-    const size_t smem_tc = sizeof(float) * ((size_t)ta.total_w + (size_t)tc::WARPS * 2 * 16 * tc::RS);
-    static size_t configured_tc = 0;
-    if (smem_tc > configured_tc) {
-      if (cudaFuncSetAttribute(tc::k_mlp_fwd_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tc) != cudaSuccess) return cnb_check_launch("mlp_fwd_tc attr");
-      configured_tc = smem_tc;
-    }
-    const int64_t nt16 = (n + 15) / 16;
-    const int64_t want = (nt16 + tc::WARPS - 1) / tc::WARPS;
-    const int grid_tc = (int)min(want, (int64_t)cnb_num_sms() * 2);
-    tc::k_mlp_fwd_tc<<<grid_tc, tc::THREADS, smem_tc, stream>>>(ta, x, x_stride, n, y, hidden);
-    return cnb_check_launch("mlp_fwd_tc");
-  }
-  const size_t smem = sizeof(float) * ((size_t)a.total_w + 2 * TILE * ROW);
+  const size_t smem = sizeof(float) * ((size_t)a.total_w + (size_t)tc::WARPS * 2 * 16 * tc::RS);
   static size_t configured = 0;
   if (smem > configured) {
-    if (cudaFuncSetAttribute(k_mlp_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return cnb_check_launch("mlp_fwd attr");
+    if (cudaFuncSetAttribute(tc::k_mlp_fwd_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return cnb_check_launch("mlp_fwd_tc attr");
     configured = smem;
   }
-  const int64_t ntiles = (n + TILE - 1) / TILE;
-  const int grid = (int)min(ntiles, (int64_t)cnb_num_sms() * 2);
-  k_mlp_fwd<<<grid, TILE, smem, stream>>>(a, x, x_stride, n, y, hidden);
-  return cnb_check_launch("mlp_fwd");
+  const int64_t nt16 = (n + 15) / 16;
+  const int64_t want = (nt16 + tc::WARPS - 1) / tc::WARPS;
+  const int grid = (int)min(want, (int64_t)cnb_num_sms() * 2);
+  tc::k_mlp_fwd_tc<<<grid, tc::THREADS, smem, stream>>>(a, x, x_stride, n, y, hidden);
+  return cnb_check_launch("mlp_fwd_tc");
 }
 
 extern "C" int cnb_mlp_bwd(const cnb_mlp* m, const float* x, int64_t x_stride, const float* hidden, const float* y, const float* dy, int64_t n,
@@ -754,41 +472,27 @@ extern "C" int cnb_mlp_bwd(const cnb_mlp* m, const float* x, int64_t x_stride, c
     for (int l = 0; l < m->num_layers; ++l) CNB_REQUIRE(m->W[l] != nullptr, "mlp_bwd: null W for layer %d", l);
     return n == 0 ? CNB_OK : cnb_mlp_wide_bwd(m, x, x_stride, hidden, y, dy, n, dx, dx_stride, stream);
   }
-  MlpArgs a;
-  int rc = make_args(m, a);
+  tc::Args a;
+  int rc = tc::make_args(m, a);
   if (rc) return rc;
   CNB_REQUIRE(n >= 0 && (n == 0 || (x && dy)), "mlp_bwd: null x/dy");
   CNB_REQUIRE(a.nl == 1 || hidden != nullptr, "mlp_bwd: hidden activations required for %d layers", a.nl);
   CNB_REQUIRE(a.act == CNB_ACT_NONE || y != nullptr, "mlp_bwd: forward output required for the output activation");
   CNB_REQUIRE(dx == nullptr || dx_stride >= a.dims[0], "mlp_bwd: dx_stride too small");
   if (n == 0) return CNB_OK;
-  if (use_tc()) {
-    tc::Args ta;
-    tc::make(a, ta);
-    const size_t tiles = 3 * (size_t)tc::ROWS * tc::RS;
-    const bool presplit = sizeof(float) * (3 * (size_t)ta.total_w + tiles) <= 232448;   // W hi, dW, W lo + three activation tiles
-    const size_t smem_tc = sizeof(float) * ((presplit ? 3 : 2) * (size_t)ta.total_w + tiles);
-    static size_t configured_tc[2] = {0, 0};
-    if (smem_tc > configured_tc[presplit]) {
-      const cudaError_t e = presplit ? cudaFuncSetAttribute(tc::k_mlp_bwd_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tc)
-                                     : cudaFuncSetAttribute(tc::k_mlp_bwd_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tc);
-      if (e != cudaSuccess) return cnb_check_launch("mlp_bwd_tc attr");
-      configured_tc[presplit] = smem_tc;
-    }
-    const int64_t nt = (n + tc::ROWS - 1) / tc::ROWS;
-    const int grid_tc = (int)min(nt, (int64_t)cnb_num_sms());
-    if (presplit) tc::k_mlp_bwd_tc<true><<<grid_tc, tc::THREADS, smem_tc, stream>>>(ta, x, x_stride, hidden, y, dy, n, dx, dx_stride);
-    else tc::k_mlp_bwd_tc<false><<<grid_tc, tc::THREADS, smem_tc, stream>>>(ta, x, x_stride, hidden, y, dy, n, dx, dx_stride);
-    return cnb_check_launch("mlp_bwd_tc");
+  const size_t tiles = 3 * (size_t)tc::ROWS * tc::RS;
+  const bool presplit = sizeof(float) * (3 * (size_t)a.total_w + tiles) <= 232448;   // W hi, dW, W lo + three activation tiles
+  const size_t smem = sizeof(float) * ((presplit ? 3 : 2) * (size_t)a.total_w + tiles);
+  static size_t configured[2] = {0, 0};
+  if (smem > configured[presplit]) {
+    const cudaError_t e = presplit ? cudaFuncSetAttribute(tc::k_mlp_bwd_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                                   : cudaFuncSetAttribute(tc::k_mlp_bwd_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return cnb_check_launch("mlp_bwd_tc attr");
+    configured[presplit] = smem;
   }
-  const size_t smem = sizeof(float) * (2 * (size_t)a.total_w + 3 * TILE * ROW);
-  static size_t configured = 0;
-  if (smem > configured) {
-    if (cudaFuncSetAttribute(k_mlp_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return cnb_check_launch("mlp_bwd attr");
-    configured = smem;
-  }
-  const int64_t ntiles = (n + TILE - 1) / TILE;
-  const int grid = (int)min(ntiles, (int64_t)cnb_num_sms());
-  k_mlp_bwd<<<grid, TILE, smem, stream>>>(a, x, x_stride, hidden, y, dy, n, dx, dx_stride);
-  return cnb_check_launch("mlp_bwd");
+  const int64_t nt = (n + tc::ROWS - 1) / tc::ROWS;
+  const int grid = (int)min(nt, (int64_t)cnb_num_sms());
+  if (presplit) tc::k_mlp_bwd_tc<true><<<grid, tc::THREADS, smem, stream>>>(a, x, x_stride, hidden, y, dy, n, dx, dx_stride);
+  else tc::k_mlp_bwd_tc<false><<<grid, tc::THREADS, smem, stream>>>(a, x, x_stride, hidden, y, dy, n, dx, dx_stride);
+  return cnb_check_launch("mlp_bwd_tc");
 }

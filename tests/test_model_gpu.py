@@ -568,21 +568,3 @@ def test_in_step_camera_optimizer_matches_the_autograd_route(dev, precision):
         assert a.abs().max().item() > 0
     pg = gb["camera_opt"][: num_images * 6].view(num_images, 6)
     assert float(pg[0, :3].abs().max()) > 0 and torch.isfinite(pg).all()
-
-
-@pytest.mark.parametrize("switch", ["CNB_FIELD_BWD=mma", "CNB_FIELD_BWD=umma", "CNB_FIELD_BWD_FUSED=1"])
-def test_field_backward_alternative_kernels(switch):
-    """The default mixed-precision field backward is the all-tcgen05 kernel (csrc/field_mixed_bwd_tc5.cu).  Its measured alternatives -- the
-    round-1 mma.sync kernel, that kernel with the dW contraction on tcgen05, and the tcgen05 kernel with the table scatter fused in -- pass the
-    same gradient-parity tests.  The switches are read once per process, hence the subprocess."""
-    import subprocess
-    import sys
-
-    k, v = switch.split("=")
-    env = dict(os.environ, **{k: v})
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_model_gpu.py"), "-m", "gpu", "-q", "-x", "-k",
-                          "test_field_backward_mixed_precision or test_train_step_ray_gradients_and_camera_optimizer"],
-                         env=env, capture_output=True, text=True, timeout=300)
-    assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-2000:]
-    assert "passed" in res.stdout
