@@ -101,6 +101,11 @@ class Camera(C.Structure):
                 ("width", C.c_int32), ("height", C.c_int32)]
 
 
+class Lens(C.Structure):
+    """cnb_lens: nerfstudio's distortion_params order."""
+    _fields_ = [("k1", C.c_float), ("k2", C.c_float), ("k3", C.c_float), ("k4", C.c_float), ("p1", C.c_float), ("p2", C.c_float)]
+
+
 class ImageSet(C.Structure):
     _fields_ = [("images_u8", C.c_void_p), ("images_f32", C.c_void_p), ("masks_u8", C.c_void_p), ("cameras", C.c_void_p),
                 ("num_images", C.c_int32), ("height", C.c_int32), ("width", C.c_int32)]
@@ -240,14 +245,17 @@ SIGNATURES = {
     "cnb_density_field_bwd_rays": (C.c_int, [C.POINTER(DensityField), C.POINTER(Samples), _P, _P, _P, _P, _P]),
     "cnb_field_bwd_rays": (C.c_int, [C.POINTER(Field), C.POINTER(Samples), _P, _P, _P, _P, _P, _P, _P, _P]),
     "cnb_generate_rays": (C.c_int, [C.POINTER(Camera), _P, _I64, C.POINTER(_F), _P, _P, _P, _P, _P, _P, _P]),
+    "cnb_generate_rays_lens": (C.c_int, [C.POINTER(Camera), C.POINTER(Lens), _P, _I64, C.POINTER(_F), _P, _P, _P, _P, _P, _P, _P]),
     "cnb_camera_opt_apply": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P, _P, _P]),
     "cnb_camera_opt_bwd": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I32, _F, _F, _F, _P, _P, _P, _P]),
     "cnb_extract_points_scratch_ints": (_I64, [_I64]),
     "cnb_extract_points": (C.c_int, [_P, _P, _P, _P, _P, _I64, C.POINTER(_F), C.c_int32, _F, _P, _P, _P, _I64, _P, _P, _P, _P]),
     "cnb_generate_rays_boxes": (C.c_int, [C.POINTER(Camera), _P, C.c_int32, _I64, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "cnb_generate_rays_boxes_lens": (C.c_int, [C.POINTER(Camera), C.POINTER(Lens), _P, C.c_int32, _I64, _P, _P, _P, _P, _P, _P, _P, _P]),
     "cnb_projection_scatter": (C.c_int, [_P, _P, _P, _I64, _F, _P, _P, _P]),
     "cnb_volume_face_rays": (C.c_int, [_F, _F, C.c_int32, _F, _F, C.c_int32, _F, C.POINTER(_F), _F, _I64, _I64, _P, _P, _P, _P, _P]),
     "cnb_sample_train_batch": (C.c_int, [C.POINTER(ImageSet), _P, _I64, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "cnb_sample_train_batch_lens": (C.c_int, [C.POINTER(ImageSet), _P, _P, _I64, _P, _P, _P, _P, _P, _P, _P, _P]),
     "cnb_sample_spaced": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I64, _I32, _P, _P, _P]),
     "cnb_sample_spaced_collide": (C.c_int, [_P, _P, _F, _F, _P, _P, _I32, _I32, _I64, _I32, _P, _P, _P, _P, _P]),
     "cnb_sample_pdf": (C.c_int, [_P, _F, _P, _P, _P, _I32, _P, _P, _I32, _I64, _I32, _I32, _F, _F, _P, _P, _P, _P]),

@@ -7,12 +7,13 @@
 //  * cnb_generate_rays_boxes  -- fruit_nerf.py:281-288 for ALL k sub-cluster boxes of a super-cluster at once: one pass over the camera's
 //    pixels builds each ray once, slab-tests it against every box and appends the hits (ray, near, far, box * npix + pixel) to one compacted
 //    list -- one launch and one count read-back per (super-cluster, camera) instead of k full-image ray bundles, k masks and 2 k syncs.
+//    cnb_generate_rays_boxes_lens undistorts the ray before the slab tests and the pixel-area offsets on the first hit (lens.cuh).
 //  * cnb_projection_scatter   -- fruit_nerf.py:296-315: semantics of the hit rays back into the k un-occluded images and, where the opacity
 //    accumulated in front of the box is below 0.5, into the k "visible" images, quantised like torchvision's save_image (x * 255 + 0.5,
 //    clamped, truncated) -- the pixels stay on the device until the PNG encoder wants them.
 //  * cnb_volume_face_rays     -- data/fruit_datamanager.py:71-120 + components/ray_generators.py:46-66 (volumetric export): the regular
 //    grid of orthographic rays on the z_min face of the export box, torch.linspace's two-sided formula evaluated per thread.
-#include "cnb_common.cuh"
+#include "lens.cuh"
 
 namespace {
 
@@ -119,9 +120,12 @@ __device__ __forceinline__ void box_dir_of(const BoxRayArgs& a, float u, float v
   dx = __fdiv_rn(dx, n); dy = __fdiv_rn(dy, n); dz = __fdiv_rn(dz, n);
 }
 
+// The lens is the last parameter so that the LENS = false instantiation reads every other parameter at the offsets it always had.
+template <bool LENS>
 __global__ void __launch_bounds__(256) k_generate_rays_boxes(const __grid_constant__ BoxRayArgs a, int64_t capacity, float* __restrict__ origins,
                                                              float* __restrict__ directions, float* __restrict__ pixel_area, float* __restrict__ nears,
-                                                             float* __restrict__ fars, int32_t* __restrict__ tags, int32_t* __restrict__ count) {
+                                                             float* __restrict__ fars, int32_t* __restrict__ tags, int32_t* __restrict__ count,
+                                                             const __grid_constant__ cnb_lens lens) {
   const int64_t npix = (int64_t)a.width * a.height;
   const int64_t nround = (npix + 31) / 32 * 32;
   const int lane = threadIdx.x & 31;
@@ -129,7 +133,9 @@ __global__ void __launch_bounds__(256) k_generate_rays_boxes(const __grid_consta
     const bool in = i < npix;
     const int py = (int)((in ? i : 0) / a.width), px = (int)((in ? i : 0) - (int64_t)py * a.width);
     const float y = (float)py + 0.5f, x = (float)px + 0.5f;
-    const float u = __fdiv_rn(__fsub_rn(x, a.cx), a.fx), v = -__fdiv_rn(__fsub_rn(y, a.cy), a.fy);
+    const float u0 = __fdiv_rn(__fsub_rn(x, a.cx), a.fx), v0 = -__fdiv_rn(__fsub_rn(y, a.cy), a.fy);
+    float u = u0, v = v0;
+    if (LENS) lens_undistort(lens, u, v);
     float dx, dy, dz;
     box_dir_of(a, u, v, dx, dy, dz);
     float area = -1.0f;  // computed on the first hit only
@@ -157,8 +163,16 @@ __global__ void __launch_bounds__(256) k_generate_rays_boxes(const __grid_consta
       if (area < 0.0f) {
         const float ux = __fdiv_rn(__fadd_rn(__fsub_rn(x, a.cx), 1.0f), a.fx), vy = -__fdiv_rn(__fadd_rn(__fsub_rn(y, a.cy), 1.0f), a.fy);
         float ex, ey, ez, gx, gy, gz;
-        box_dir_of(a, ux, v, ex, ey, ez);
-        box_dir_of(a, u, vy, gx, gy, gz);
+        if (LENS) {
+          float u1 = ux, v1 = v0, u2 = u0, v2 = vy;
+          lens_undistort(lens, u1, v1);
+          lens_undistort(lens, u2, v2);
+          box_dir_of(a, u1, v1, ex, ey, ez);
+          box_dir_of(a, u2, v2, gx, gy, gz);
+        } else {
+          box_dir_of(a, ux, v, ex, ey, ez);
+          box_dir_of(a, u, vy, gx, gy, gz);
+        }
         const float sx = sqrtf((dx - ex) * (dx - ex) + (dy - ey) * (dy - ey) + (dz - ez) * (dz - ez));
         const float sy = sqrtf((dx - gx) * (dx - gx) + (dy - gy) * (dy - gy) + (dz - gz) * (dz - gz));
         area = sx * sy;
@@ -249,8 +263,9 @@ extern "C" int cnb_extract_points(const float* origins, const float* directions,
   return cnb_check_launch("extract_points write");
 }
 
-extern "C" int cnb_generate_rays_boxes(const cnb_camera* cam, const float* boxes, int32_t num_boxes, int64_t capacity, float* origins, float* directions,
-                                       float* pixel_area, float* nears, float* fars, int32_t* tags, int32_t* count, cnb_stream_t stream) {
+extern "C" int cnb_generate_rays_boxes_lens(const cnb_camera* cam, const cnb_lens* lens, const float* boxes, int32_t num_boxes, int64_t capacity,
+                                            float* origins, float* directions, float* pixel_area, float* nears, float* fars, int32_t* tags,
+                                            int32_t* count, cnb_stream_t stream) {
   CNB_REQUIRE(cam && boxes && num_boxes >= 1 && capacity >= 0, "generate_rays_boxes: null camera / boxes");
   CNB_REQUIRE(origins && directions && pixel_area && nears && fars && tags && count, "generate_rays_boxes: null output");
   CNB_REQUIRE(cam->width > 0 && cam->height > 0 && cam->fx != 0.0f && cam->fy != 0.0f, "generate_rays_boxes: bad intrinsics");
@@ -262,8 +277,17 @@ extern "C" int cnb_generate_rays_boxes(const cnb_camera* cam, const float* boxes
   }
   a.fx = cam->fx; a.fy = cam->fy; a.cx = cam->cx; a.cy = cam->cy; a.width = cam->width; a.height = cam->height;
   a.boxes = boxes; a.k = num_boxes;
-  k_generate_rays_boxes<<<grid_cap((int64_t)cam->width * cam->height, 256, 8), 256, 0, stream>>>(a, capacity, origins, directions, pixel_area, nears, fars, tags, count);
+  const int blocks = grid_cap((int64_t)cam->width * cam->height, 256, 8);
+  if (lens_active(lens))
+    k_generate_rays_boxes<true><<<blocks, 256, 0, stream>>>(a, capacity, origins, directions, pixel_area, nears, fars, tags, count, *lens);
+  else
+    k_generate_rays_boxes<false><<<blocks, 256, 0, stream>>>(a, capacity, origins, directions, pixel_area, nears, fars, tags, count, cnb_lens{});
   return cnb_check_launch("generate_rays_boxes");
+}
+
+extern "C" int cnb_generate_rays_boxes(const cnb_camera* cam, const float* boxes, int32_t num_boxes, int64_t capacity, float* origins, float* directions,
+                                       float* pixel_area, float* nears, float* fars, int32_t* tags, int32_t* count, cnb_stream_t stream) {
+  return cnb_generate_rays_boxes_lens(cam, nullptr, boxes, num_boxes, capacity, origins, directions, pixel_area, nears, fars, tags, count, stream);
 }
 
 extern "C" int cnb_projection_scatter(const int32_t* tags, const float* semantics, const float* front_opacity, int64_t n, float occlusion_threshold,

@@ -4,7 +4,9 @@
 // One thread per pixel: nerfstudio Cameras._generate_rays_from_coords (perspective, no distortion; pixel centres at +0.5;
 // OpenGL camera axes; pixel_area from the two neighbouring-pixel directions) fused with nerfstudio/utils/math.py
 // intersect_aabb (slab test; misses get nears = fars = 1e10) and an optional count of the rays that hit the box.
-#include "cnb_common.cuh"
+// LENS = true (cnb_generate_rays_lens) undistorts the three normalised coordinates of every ray first (lens.cuh), as nerfstudio does
+// for a camera with non-zero distortion_params; LENS = false is the pinhole kernel, which ignores the trailing lens argument.
+#include "lens.cuh"
 
 namespace {
 
@@ -27,21 +29,34 @@ __device__ __forceinline__ void dir_of(const RayGenArgs& a, float u, float v, fl
   dx = __fdiv_rn(dx, n); dy = __fdiv_rn(dy, n); dz = __fdiv_rn(dz, n);
 }
 
+// The lens is the last parameter so that the LENS = false instantiation reads every other parameter at the offsets it always had.
+template <bool LENS>
 __global__ void __launch_bounds__(256) k_generate_rays(const __grid_constant__ RayGenArgs a, const int32_t* __restrict__ pixel_yx, int64_t n,
                                                        float* __restrict__ origins, float* __restrict__ directions, float* __restrict__ pixel_area,
-                                                       float* __restrict__ nears, float* __restrict__ fars, int32_t* __restrict__ valid_count) {
+                                                       float* __restrict__ nears, float* __restrict__ fars, int32_t* __restrict__ valid_count,
+                                                       const __grid_constant__ cnb_lens lens) {
   int local_valid = 0;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     int py, px;
     if (pixel_yx) { py = __ldg(pixel_yx + 2 * i); px = __ldg(pixel_yx + 2 * i + 1); }
     else { py = (int)(i / a.width); px = (int)(i - (int64_t)py * a.width); }
     const float y = (float)py + 0.5f, x = (float)px + 0.5f;
-    const float u = __fdiv_rn(__fsub_rn(x, a.cx), a.fx), v = -__fdiv_rn(__fsub_rn(y, a.cy), a.fy);
+    float u = __fdiv_rn(__fsub_rn(x, a.cx), a.fx), v = -__fdiv_rn(__fsub_rn(y, a.cy), a.fy);
     const float ux = __fdiv_rn(__fadd_rn(__fsub_rn(x, a.cx), 1.0f), a.fx), vy = -__fdiv_rn(__fadd_rn(__fsub_rn(y, a.cy), 1.0f), a.fy);
+    // the offset coordinates share one of their two components with the ray's before undistortion, not after
+    float u1 = ux, v1 = v, u2 = u, v2 = vy;
+    if (LENS) {
+      lens_undistort(lens, u, v);
+      if (pixel_area) { lens_undistort(lens, u1, v1); lens_undistort(lens, u2, v2); }
+    }
     float dx, dy, dz, ex, ey, ez, gx, gy, gz;
     dir_of(a, u, v, dx, dy, dz);
-    dir_of(a, ux, v, ex, ey, ez);
-    dir_of(a, u, vy, gx, gy, gz);
+    if (LENS) {
+      if (pixel_area) { dir_of(a, u1, v1, ex, ey, ez); dir_of(a, u2, v2, gx, gy, gz); }
+    } else {
+      dir_of(a, ux, v, ex, ey, ez);
+      dir_of(a, u, vy, gx, gy, gz);
+    }
     origins[3 * i] = a.t[0]; origins[3 * i + 1] = a.t[1]; origins[3 * i + 2] = a.t[2];
     directions[3 * i] = dx; directions[3 * i + 1] = dy; directions[3 * i + 2] = dz;
     if (pixel_area) {
@@ -73,10 +88,8 @@ __global__ void __launch_bounds__(256) k_generate_rays(const __grid_constant__ R
   }
 }
 
-}  // namespace
-
-extern "C" int cnb_generate_rays(const cnb_camera* cam, const int32_t* pixel_yx, int64_t n, const float* aabb, float* origins, float* directions,
-                                 float* pixel_area, float* nears, float* fars, int32_t* valid_count, cnb_stream_t stream) {
+int launch_generate_rays(const cnb_camera* cam, const cnb_lens* lens, const int32_t* pixel_yx, int64_t n, const float* aabb, float* origins,
+                         float* directions, float* pixel_area, float* nears, float* fars, int32_t* valid_count, cnb_stream_t stream) {
   CNB_REQUIRE(cam != nullptr && n >= 0, "generate_rays: null camera / negative count");
   if (n == 0) return CNB_OK;
   CNB_REQUIRE(origins && directions, "generate_rays: null outputs");
@@ -94,6 +107,22 @@ extern "C" int cnb_generate_rays(const cnb_camera* cam, const int32_t* pixel_yx,
   int64_t blocks = (n + 255) / 256;
   const int64_t cap = (int64_t)cnb_num_sms() * 16;
   if (blocks > cap) blocks = cap;
-  k_generate_rays<<<(int)blocks, 256, 0, stream>>>(a, pixel_yx, n, origins, directions, pixel_area, nears, fars, valid_count);
+  if (lens_active(lens))
+    k_generate_rays<true><<<(int)blocks, 256, 0, stream>>>(a, pixel_yx, n, origins, directions, pixel_area, nears, fars, valid_count, *lens);
+  else
+    k_generate_rays<false><<<(int)blocks, 256, 0, stream>>>(a, pixel_yx, n, origins, directions, pixel_area, nears, fars, valid_count, cnb_lens{});
   return cnb_check_launch("generate_rays");
+}
+
+}  // namespace
+
+extern "C" int cnb_generate_rays(const cnb_camera* cam, const int32_t* pixel_yx, int64_t n, const float* aabb, float* origins, float* directions,
+                                 float* pixel_area, float* nears, float* fars, int32_t* valid_count, cnb_stream_t stream) {
+  return launch_generate_rays(cam, nullptr, pixel_yx, n, aabb, origins, directions, pixel_area, nears, fars, valid_count, stream);
+}
+
+extern "C" int cnb_generate_rays_lens(const cnb_camera* cam, const cnb_lens* lens, const int32_t* pixel_yx, int64_t n, const float* aabb,
+                                      float* origins, float* directions, float* pixel_area, float* nears, float* fars, int32_t* valid_count,
+                                      cnb_stream_t stream) {
+  return launch_generate_rays(cam, lens, pixel_yx, n, aabb, origins, directions, pixel_area, nears, fars, valid_count, stream);
 }

@@ -6,10 +6,11 @@
 //                                                                 Cameras.generate_rays(camera_indices=c, coords=...)
 // With the images resident in HBM (300 x 1080p: 1.9 GB as uint8 RGB + 0.6 GB of masks) one thread per ray does index -> pixel gather ->
 // per-camera pinhole ray -> pixel area; the outputs are exactly the tensors cnb_train_step reads (origins, directions, camera indices,
-// image, fruit_mask), so a training step needs no host batch at all.  Ray arithmetic = k_generate_rays (raygen.cu), op for op.
+// image, fruit_mask), so a training step needs no host batch at all.  Ray arithmetic = k_generate_rays (raygen.cu), op for op,
+// including the per-camera lens undistortion of cnb_sample_train_batch_lens (LENS = true; lens.cuh).
 #include <cstddef>
 
-#include "cnb_common.cuh"
+#include "lens.cuh"
 
 namespace {
 
@@ -37,10 +38,13 @@ __device__ __forceinline__ int scaled_index(float rnd, int extent) {
   return min(max(v, 0), extent - 1);
 }
 
+// lenses [N] (device) is the last parameter so that the LENS = false instantiation reads every other parameter where it always did
+template <bool LENS>
 __global__ void __launch_bounds__(256) k_sample_train_batch(const __grid_constant__ TrainBatchArgs a, const float* __restrict__ rand3, int64_t R,
                                                             int32_t* __restrict__ indices, float* __restrict__ origins, float* __restrict__ directions,
                                                             float* __restrict__ pixel_area, int32_t* __restrict__ camera_indices,
-                                                            float* __restrict__ image, float* __restrict__ fruit_mask) {
+                                                            float* __restrict__ image, float* __restrict__ fruit_mask,
+                                                            const cnb_lens* __restrict__ lenses) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < R; i += (int64_t)gridDim.x * blockDim.x) {
     const int c = scaled_index(__ldg(rand3 + 3 * i), a.N);
     const int py = scaled_index(__ldg(rand3 + 3 * i + 1), a.H);
@@ -71,12 +75,27 @@ __global__ void __launch_bounds__(256) k_sample_train_batch(const __grid_constan
     }
     const float fx = __ldg(cam + 12), fy = __ldg(cam + 13), cx = __ldg(cam + 14), cy = __ldg(cam + 15);
     const float y = (float)py + 0.5f, x = (float)px + 0.5f;
-    const float u = __fdiv_rn(__fsub_rn(x, cx), fx), v = -__fdiv_rn(__fsub_rn(y, cy), fy);
+    float u = __fdiv_rn(__fsub_rn(x, cx), fx), v = -__fdiv_rn(__fsub_rn(y, cy), fy);
     const float ux = __fdiv_rn(__fadd_rn(__fsub_rn(x, cx), 1.0f), fx), vy = -__fdiv_rn(__fadd_rn(__fsub_rn(y, cy), 1.0f), fy);
     float dx, dy, dz, ex, ey, ez, gx, gy, gz;
-    camera_direction(r, u, v, dx, dy, dz);
-    camera_direction(r, ux, v, ex, ey, ez);
-    camera_direction(r, u, vy, gx, gy, gz);
+    if (LENS) {
+      // the three coordinates are undistorted independently (the offsets share one component with the ray's only before it)
+      const float* lp = reinterpret_cast<const float*>(lenses + c);
+      const cnb_lens l = {__ldg(lp), __ldg(lp + 1), __ldg(lp + 2), __ldg(lp + 3), __ldg(lp + 4), __ldg(lp + 5)};
+      float u1 = ux, v1 = v, u2 = u, v2 = vy;
+      lens_undistort(l, u, v);
+      camera_direction(r, u, v, dx, dy, dz);
+      if (pixel_area) {
+        lens_undistort(l, u1, v1);
+        lens_undistort(l, u2, v2);
+        camera_direction(r, u1, v1, ex, ey, ez);
+        camera_direction(r, u2, v2, gx, gy, gz);
+      }
+    } else {
+      camera_direction(r, u, v, dx, dy, dz);
+      camera_direction(r, ux, v, ex, ey, ez);
+      camera_direction(r, u, vy, gx, gy, gz);
+    }
     origins[3 * i] = t[0]; origins[3 * i + 1] = t[1]; origins[3 * i + 2] = t[2];
     directions[3 * i] = dx; directions[3 * i + 1] = dy; directions[3 * i + 2] = dz;
     if (pixel_area) {
@@ -87,10 +106,8 @@ __global__ void __launch_bounds__(256) k_sample_train_batch(const __grid_constan
   }
 }
 
-}  // namespace
-
-extern "C" int cnb_sample_train_batch(const cnb_image_set* set, const float* rand3, int64_t R, int32_t* indices, float* origins, float* directions,
-                                      float* pixel_area, int32_t* camera_indices, float* image, float* fruit_mask, cnb_stream_t stream) {
+int launch_sample_train_batch(const cnb_image_set* set, const cnb_lens* lenses, const float* rand3, int64_t R, int32_t* indices, float* origins,
+                              float* directions, float* pixel_area, int32_t* camera_indices, float* image, float* fruit_mask, cnb_stream_t stream) {
   CNB_REQUIRE(set != nullptr && R >= 0, "sample_train_batch: null image set / negative count");
   if (R == 0) return CNB_OK;
   CNB_REQUIRE(rand3 && origins && directions, "sample_train_batch: null rand / ray outputs");
@@ -104,6 +121,25 @@ extern "C" int cnb_sample_train_batch(const cnb_image_set* set, const float* ran
   int64_t blocks = (R + 255) / 256;
   const int64_t cap = (int64_t)cnb_num_sms() * 16;
   if (blocks > cap) blocks = cap;
-  k_sample_train_batch<<<(int)blocks, 256, 0, stream>>>(a, rand3, R, indices, origins, directions, pixel_area, camera_indices, image, fruit_mask);
+  static_assert(sizeof(cnb_lens) == 24, "k_sample_train_batch reads cnb_lens as 6 floats");
+  if (lenses)
+    k_sample_train_batch<true><<<(int)blocks, 256, 0, stream>>>(a, rand3, R, indices, origins, directions, pixel_area, camera_indices, image, fruit_mask,
+                                                                lenses);
+  else
+    k_sample_train_batch<false><<<(int)blocks, 256, 0, stream>>>(a, rand3, R, indices, origins, directions, pixel_area, camera_indices, image, fruit_mask,
+                                                                 nullptr);
   return cnb_check_launch("sample_train_batch");
+}
+
+}  // namespace
+
+extern "C" int cnb_sample_train_batch(const cnb_image_set* set, const float* rand3, int64_t R, int32_t* indices, float* origins, float* directions,
+                                      float* pixel_area, int32_t* camera_indices, float* image, float* fruit_mask, cnb_stream_t stream) {
+  return launch_sample_train_batch(set, nullptr, rand3, R, indices, origins, directions, pixel_area, camera_indices, image, fruit_mask, stream);
+}
+
+extern "C" int cnb_sample_train_batch_lens(const cnb_image_set* set, const cnb_lens* lenses, const float* rand3, int64_t R, int32_t* indices,
+                                           float* origins, float* directions, float* pixel_area, int32_t* camera_indices, float* image, float* fruit_mask,
+                                           cnb_stream_t stream) {
+  return launch_sample_train_batch(set, lenses, rand3, R, indices, origins, directions, pixel_area, camera_indices, image, fruit_mask, stream);
 }

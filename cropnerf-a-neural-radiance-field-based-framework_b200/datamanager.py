@@ -5,7 +5,8 @@ The reference draws a batch as ``batch = train_pixel_sampler.sample(image_batch)
 ``ray_bundle = train_ray_generator(batch["indices"])`` (nerfstudio ``RayGenerator``: pixel centres -> ``Cameras.generate_rays``).
 Here the images of the split stay in HBM (uint8 RGB: 300 x 1080p = 1.9 GB, masks 0.6 GB) and ``cnb_sample_train_batch``
 (``csrc/train_batch.cu``) does index -> pixel gather -> per-camera pinhole ray -> pixel area, one thread per ray, writing exactly
-the tensors the training step reads.  SURVEY.md section 8, "next" row f1 (pixel sampler).
+the tensors the training step reads.  SURVEY.md section 8, "next" row f1 (pixel sampler).  Cameras with OPENCV lens distortion
+(nerfstudio ``distortion_params``) get nerfstudio's undistortion in the same kernel (``cnb_sample_train_batch_lens``).
 
 Parity: ``tests/test_train_batch_gpu.py`` (indices and gathered pixels bit-exact against the oracle, uint8 and float32 storage);
 ``bench.py``'s end-to-end leg ``e2e_device_batches`` trains from it (images resident in HBM, no host ray traffic at all).
@@ -19,6 +20,7 @@ import torch
 from torch import Tensor
 
 from . import _lib as L
+from .export import cameras_from_nerfstudio, check_perspective, lens_values
 from .rays import RayBundle
 
 
@@ -26,9 +28,13 @@ class DeviceTrainBatches:
     """``next_train(step) -> (RayBundle, batch)`` with nerfstudio's batch keys (``image``, ``fruit_mask``, ``indices``).
 
     ``images``: ``[N,H,W,3]`` uint8 (value / 255 is the float image ``cotton_dataset.py`` produces) or float32; ``fruit_masks``:
-    ``[N,H,W]`` uint8 / bool (non-zero = fruit) or None; ``cameras``: N objects with ``c2w`` ``[3,4]``, ``fx, fy, cx, cy``
-    (``export.PinholeCamera`` or a nerfstudio ``Cameras`` row).  ``rand_fn(shape, device)`` is injectable so that tests feed the
-    oracle the same numbers; default ``torch.rand`` on the device with this object's generator."""
+    ``[N,H,W]`` uint8 / bool (non-zero = fruit) or None.  ``cameras``: either N objects with ``c2w`` ``[3,4]``, ``fx, fy, cx, cy``
+    and optionally ``distortion_params`` (6 values, nerfstudio order) and ``camera_type`` (``export.PinholeCamera``), or a
+    nerfstudio ``Cameras`` batch of N cameras, which is read through ``export.cameras_from_nerfstudio`` (``camera_to_worlds``,
+    intrinsics, ``distortion_params``, ``camera_type``).  Only perspective cameras are accepted; any other ``camera_type`` raises
+    ``ValueError``.  If some camera has non-zero distortion, the ``[N,6]`` parameters are uploaded once here and every batch is
+    undistorted as nerfstudio's ``RayGenerator`` does.  ``rand_fn(shape, device)`` is injectable so that tests feed the oracle
+    the same numbers; default ``torch.rand`` on the device with this object's generator."""
 
     def __init__(self, images: Tensor, fruit_masks: Optional[Tensor], cameras: Sequence, num_rays_per_batch: int = 4096, device="cuda",
                  seed: int = 0, rand_fn=None):
@@ -38,6 +44,8 @@ class DeviceTrainBatches:
         if images.dim() != 4 or images.shape[-1] != 3 or images.dtype not in (torch.uint8, torch.float32):
             raise ValueError(f"images must be [N,H,W,3] uint8 or float32, got {tuple(images.shape)} {images.dtype}")
         n, h, w = images.shape[:3]
+        if hasattr(cameras, "camera_to_worlds"):         # a nerfstudio Cameras batch
+            cameras = cameras_from_nerfstudio(cameras)
         if len(cameras) != n:
             raise ValueError(f"{len(cameras)} cameras for {n} images")
         self.device = dev
@@ -48,7 +56,12 @@ class DeviceTrainBatches:
                 raise ValueError(f"fruit_masks must be [N,H,W] = {(n, h, w)}, got {tuple(fruit_masks.shape)}")
             self.masks = (fruit_masks != 0).to(dev, torch.uint8).contiguous()
         cam_host = (L.Camera * n)()
+        lenses = torch.zeros((n, 6), dtype=torch.float32)
         for i, cam in enumerate(cameras):
+            check_perspective(getattr(cam, "camera_type", None), "DeviceTrainBatches")
+            dist = lens_values(getattr(cam, "distortion_params", None))
+            if dist is not None:
+                lenses[i] = torch.tensor(dist, dtype=torch.float32)
             m = torch.as_tensor(cam.c2w).detach().cpu().float().reshape(-1)[:12].tolist()
             for k in range(12):
                 cam_host[i].c2w[k] = m[k]
@@ -56,6 +69,8 @@ class DeviceTrainBatches:
             cam_host[i].width, cam_host[i].height = int(w), int(h)
         raw = torch.frombuffer(bytearray(bytes(cam_host)), dtype=torch.uint8)
         self._cameras = raw.to(dev)                      # device array of cnb_camera records (72 bytes each)
+        # device array of cnb_lens records [N,6], only when some camera is distorted (otherwise the pinhole kernel runs)
+        self._lenses = lenses.to(dev) if bool((lenses != 0).any()) else None
         self.num_rays_per_batch = int(num_rays_per_batch)
         self.generator = torch.Generator(device=dev)
         self.generator.manual_seed(int(seed))
@@ -83,8 +98,13 @@ class DeviceTrainBatches:
         camera_indices = torch.empty((R, 1), device=dev, dtype=torch.int32)
         image = torch.empty((R, 3), device=dev, dtype=torch.float32)
         fruit_mask = torch.empty((R, 1), device=dev, dtype=torch.float32)
-        L.check(L.lib().cnb_sample_train_batch(C.byref(self._set), rand3.data_ptr(), R, indices.data_ptr(), origins.data_ptr(), directions.data_ptr(),
-                                               pixel_area.data_ptr(), camera_indices.data_ptr(), image.data_ptr(), fruit_mask.data_ptr(),
-                                               L.stream_ptr(dev)), "sample_train_batch")
+        if self._lenses is None:
+            L.check(L.lib().cnb_sample_train_batch(C.byref(self._set), rand3.data_ptr(), R, indices.data_ptr(), origins.data_ptr(), directions.data_ptr(),
+                                                   pixel_area.data_ptr(), camera_indices.data_ptr(), image.data_ptr(), fruit_mask.data_ptr(),
+                                                   L.stream_ptr(dev)), "sample_train_batch")
+        else:
+            L.check(L.lib().cnb_sample_train_batch_lens(C.byref(self._set), self._lenses.data_ptr(), rand3.data_ptr(), R, indices.data_ptr(),
+                                                        origins.data_ptr(), directions.data_ptr(), pixel_area.data_ptr(), camera_indices.data_ptr(),
+                                                        image.data_ptr(), fruit_mask.data_ptr(), L.stream_ptr(dev)), "sample_train_batch_lens")
         bundle = RayBundle(origins=origins, directions=directions, pixel_area=pixel_area, camera_indices=camera_indices)
         return bundle, {"image": image, "fruit_mask": fruit_mask, "indices": indices}

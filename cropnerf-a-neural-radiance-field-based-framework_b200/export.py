@@ -10,7 +10,9 @@ collective (SURVEY.md section 8e).
   (``fruit_nerf.py:283-315``): un-occluded semantic render of the rays hitting the box, and the opacity accumulated in
   front of the box (occluded where >= 0.5).
 * :func:`write_ply` -- ``semantics_pc.ply`` in the layout ``segmentation/segmenter.py:210`` reads (float xyz, uchar rgb).
-* :func:`generate_rays` -- device-side ``cam.generate_rays(aabb_box=...)`` (pixel -> ray -> slab test in one kernel).
+* :func:`generate_rays` -- device-side ``cam.generate_rays(aabb_box=...)`` (pixel -> ray -> slab test in one kernel), with
+  nerfstudio's OPENCV lens undistortion when the camera has non-zero ``distortion_params``.
+* :func:`cameras_from_nerfstudio` -- nerfstudio ``Cameras`` -> :class:`PinholeCamera` list (perspective only; others are refused).
 * :func:`project_clusters` -- the whole ``get_outputs_for_projections`` loop (``fruit_nerf.py:254-318``) writing the
   ``super_cluster_k/cam_j/{wo_occ,visible}_cluster_i.png`` tree ``segmentation/merger.py`` reads, sharded over ranks.
 """
@@ -149,12 +151,14 @@ def write_ply(path: str, points: Tensor, rgbs: Tensor) -> None:
 
 
 def generate_rays(c2w: Tensor, fx: float, fy: float, cx: float, cy: float, width: int, height: int, device, aabb: Optional[Tensor] = None,
-                  pixel_yx: Optional[Tensor] = None, camera_index: int = 0, count_valid: bool = False):
+                  pixel_yx: Optional[Tensor] = None, camera_index: int = 0, count_valid: bool = False, distortion_params: Optional[Tensor] = None):
     """``cam.generate_rays(camera_indices=0, keep_shape=True, aabb_box=aabb)`` (fruit_nerf.py:283) for one perspective camera
     on the device: one kernel does pixel -> direction -> normalisation -> pixel_area -> AABB slab test (``cnb_generate_rays``).
     Returns a flat RayBundle of width*height rays (or of the given integer ``pixel_yx`` [n,2]); with ``aabb`` ([2,3] or [6])
     ``nears``/``fars`` are set and misses carry 1e10 (``valid = nears < 1e10``, fruit_nerf.py:286).  ``count_valid`` also
-    returns the number of rays that hit the box as a device int32 tensor (no host sync)."""
+    returns the number of rays that hit the box as a device int32 tensor (no host sync).  ``distortion_params`` (6 values,
+    nerfstudio's ``[k1, k2, k3, k4, p1, p2]``) undistorts every pixel coordinate as nerfstudio does (``cnb_generate_rays_lens``);
+    None or all zero gives the pinhole rays."""
     import ctypes as C
 
     from . import _lib as L
@@ -181,8 +185,13 @@ def generate_rays(c2w: Tensor, fx: float, fy: float, cx: float, cy: float, width
     nears = torch.empty((n, 1), device=dev, dtype=torch.float32) if aabb is not None else None
     fars = torch.empty((n, 1), device=dev, dtype=torch.float32) if aabb is not None else None
     cnt = torch.zeros((1,), device=dev, dtype=torch.int32) if (count_valid and aabb is not None) else None
-    L.check(L.lib().cnb_generate_rays(C.byref(cam), L.ptr(pix), n, box, o.data_ptr(), d.data_ptr(), area.data_ptr(), L.ptr(nears), L.ptr(fars),
-                                      L.ptr(cnt), L.stream_ptr(dev)), "generate_rays")
+    lens = _lens_struct(distortion_params)
+    if lens is None:
+        L.check(L.lib().cnb_generate_rays(C.byref(cam), L.ptr(pix), n, box, o.data_ptr(), d.data_ptr(), area.data_ptr(), L.ptr(nears), L.ptr(fars),
+                                          L.ptr(cnt), L.stream_ptr(dev)), "generate_rays")
+    else:
+        L.check(L.lib().cnb_generate_rays_lens(C.byref(cam), C.byref(lens), L.ptr(pix), n, box, o.data_ptr(), d.data_ptr(), area.data_ptr(),
+                                               L.ptr(nears), L.ptr(fars), L.ptr(cnt), L.stream_ptr(dev)), "generate_rays_lens")
     rb = RayBundle(origins=o, directions=d, pixel_area=area, camera_indices=torch.full((n, 1), int(camera_index), device=dev, dtype=torch.int32),
                    nears=nears, fars=fars)
     return (rb, cnt) if count_valid else rb
@@ -232,7 +241,8 @@ def render_cluster_projection(model, rays: RayBundle, aabb: Tensor) -> Dict[str,
 
 @dataclass
 class PinholeCamera:
-    """What the projection loop needs of one nerfstudio ``Cameras`` entry (perspective, no distortion)."""
+    """What the projection loop needs of one nerfstudio ``Cameras`` entry: a perspective camera, optionally with OPENCV lens
+    distortion (``distortion_params``: 6 values in nerfstudio's order ``[k1, k2, k3, k4, p1, p2]``; None = none)."""
 
     c2w: Tensor  # [3,4]
     fx: float
@@ -241,6 +251,76 @@ class PinholeCamera:
     cy: float
     width: int
     height: int
+    distortion_params: Optional[Tensor] = None
+
+
+# nerfstudio cameras/cameras.py CameraType (enum auto() values); only PERSPECTIVE is generated here
+_CAMERA_TYPES = {1: "PERSPECTIVE", 2: "FISHEYE", 3: "EQUIRECTANGULAR", 4: "OMNIDIRECTIONALSTEREO_L", 5: "OMNIDIRECTIONALSTEREO_R", 6: "VR180_L",
+                 7: "VR180_R", 8: "ORTHOPHOTO", 9: "FISHEYE624"}
+_PERSPECTIVE = 1
+
+
+def check_perspective(camera_type, what: str) -> None:
+    """Raise ``ValueError`` naming the type unless every entry of ``camera_type`` (a nerfstudio ``camera_type`` tensor, a
+    ``CameraType`` member or an int; None = perspective) is ``CameraType.PERSPECTIVE``.  Other projection models are refused,
+    not rendered as pinholes."""
+    if camera_type is None:
+        return
+    values = torch.as_tensor(getattr(camera_type, "value", camera_type)).reshape(-1).tolist()
+    for v in values:
+        if int(v) != _PERSPECTIVE:
+            raise ValueError(f"{what}: camera type {_CAMERA_TYPES.get(int(v), int(v))} is not supported; only perspective cameras "
+                             "(with or without OPENCV k1..k4, p1, p2 distortion) are")
+
+
+def lens_values(distortion_params) -> Optional[List[float]]:
+    """nerfstudio ``distortion_params`` of one camera -> its 6 floats (None stays None)."""
+    if distortion_params is None:
+        return None
+    t = torch.as_tensor(distortion_params).detach().cpu().to(torch.float32).reshape(-1)
+    if t.numel() != 6:
+        raise ValueError(f"distortion_params must hold 6 values [k1, k2, k3, k4, p1, p2], got {t.numel()}")
+    return t.tolist()
+
+
+def _lens_struct(distortion_params):
+    from . import _lib as L
+
+    v = lens_values(distortion_params)
+    return None if v is None else L.Lens(*v)
+
+
+def cameras_from_nerfstudio(cameras) -> List[PinholeCamera]:
+    """nerfstudio ``Cameras`` (batch [N], or one row) -> one :class:`PinholeCamera` per camera, read by attribute name so that
+    nerfstudio need not be importable: ``camera_to_worlds`` [N,3,4], ``fx, fy, cx, cy, width, height`` [N,1],
+    ``distortion_params`` [N,6] or None, ``camera_type`` [N,1].  Raises ``ValueError`` on a camera that is not perspective
+    (fisheye, equirectangular, fisheye624, orthophoto, ...) and on unexpected shapes."""
+    c2w = torch.as_tensor(cameras.camera_to_worlds).detach().cpu().to(torch.float32)
+    single = c2w.dim() == 2
+    if single:
+        c2w = c2w[None]
+    if c2w.dim() != 3 or tuple(c2w.shape[1:]) != (3, 4):
+        raise ValueError(f"cameras.camera_to_worlds has shape {tuple(cameras.camera_to_worlds.shape)}, expected [N,3,4]")
+    n = int(c2w.shape[0])
+
+    def per_camera(name, width):
+        t = torch.as_tensor(getattr(cameras, name)).detach().cpu()
+        want = (width,) if single else (n, width)
+        if tuple(t.shape) != want:
+            raise ValueError(f"cameras.{name} has shape {tuple(t.shape)}, expected {list(want)}")
+        return t.reshape(n, width)
+
+    camera_type = getattr(cameras, "camera_type", None)
+    if camera_type is not None:
+        if isinstance(camera_type, Tensor):
+            per_camera("camera_type", 1)
+        check_perspective(camera_type, "cameras_from_nerfstudio")
+    fx, fy, cx, cy = (per_camera(k, 1).to(torch.float32) for k in ("fx", "fy", "cx", "cy"))
+    width, height = per_camera("width", 1), per_camera("height", 1)
+    dist = per_camera("distortion_params", 6).to(torch.float32) if getattr(cameras, "distortion_params", None) is not None else None
+    return [PinholeCamera(c2w=c2w[i].clone(), fx=float(fx[i, 0]), fy=float(fy[i, 0]), cx=float(cx[i, 0]), cy=float(cy[i, 0]),
+                          width=int(width[i, 0]), height=int(height[i, 0]), distortion_params=None if dist is None else dist[i].clone())
+            for i in range(n)]
 
 
 class _NumpyOnlyUnpickler(pickle.Unpickler):
@@ -345,7 +425,9 @@ def project_camera_boxes(model, cam: "PinholeCamera", boxes: Tensor, min_valid_r
     k = int(boxes_d.shape[0])
     npix = int(cam.width) * int(cam.height)
     cap = int(capacity) if capacity is not None else min(k * npix, max(npix, 1 << 21))
+    check_perspective(getattr(cam, "camera_type", None), "project_camera_boxes")
     cs = _camera_struct(cam)
+    lens = _lens_struct(getattr(cam, "distortion_params", None))
     lib = L.lib()
     while True:
         o = torch.empty((cap, 3), device=dev)
@@ -355,8 +437,9 @@ def project_camera_boxes(model, cam: "PinholeCamera", boxes: Tensor, min_valid_r
         fars = torch.empty((cap, 1), device=dev)
         tags = torch.empty((cap,), device=dev, dtype=torch.int32)
         count = torch.zeros((1,), device=dev, dtype=torch.int32)
-        L.check(lib.cnb_generate_rays_boxes(C.byref(cs), boxes_d.data_ptr(), k, cap, o.data_ptr(), d.data_ptr(), area.data_ptr(), nears.data_ptr(),
-                                            fars.data_ptr(), tags.data_ptr(), count.data_ptr(), L.stream_ptr(dev)), "generate_rays_boxes")
+        L.check(lib.cnb_generate_rays_boxes_lens(C.byref(cs), None if lens is None else C.byref(lens), boxes_d.data_ptr(), k, cap, o.data_ptr(),
+                                                 d.data_ptr(), area.data_ptr(), nears.data_ptr(), fars.data_ptr(), tags.data_ptr(), count.data_ptr(),
+                                                 L.stream_ptr(dev)), "generate_rays_boxes")
         n = int(count.item())  # the one host read-back of the pair
         if n <= cap:
             break
@@ -398,9 +481,16 @@ def project_clusters(model, cameras: Sequence[PinholeCamera], clusters: List[dic
     the ranks (no communication).  Every pair is one :func:`project_camera_boxes` call (all sub-cluster boxes of the super-cluster in one
     ray-generation pass and two batched renders); the uint8 images come down in one copy per pair and are written as
     ``super_cluster_{k}/cam_{j}/wo_occ_cluster_{i}.png`` / ``visible_cluster_{i}.png`` -- the layout segmentation/merger.py:219-333 reads.
-    ``out_dir=None`` renders without writing files (benchmarks).  Returns counters (pairs, images, rays rendered)."""
+    ``out_dir=None`` renders without writing files (benchmarks).  Returns counters (pairs, images, rays rendered).
+    ``cameras`` may also be a nerfstudio ``Cameras`` batch (see :func:`cameras_from_nerfstudio`); lens distortion is applied, and a
+    camera that is not perspective raises ``ValueError`` before anything is rendered."""
     import os
     import shutil
+
+    if hasattr(cameras, "camera_to_worlds"):
+        cameras = cameras_from_nerfstudio(cameras)
+    for cam in cameras:
+        check_perspective(getattr(cam, "camera_type", None), "project_clusters")
 
     stats = {"pairs": 0, "images": 0, "rays": 0}
     pair = 0

@@ -266,18 +266,28 @@ int cnb_interlevel_fused(const float* c, const float* w, const float* cp, const 
                          int64_t R, int32_t Sc, int32_t Sp, float grad_scale, float* loss_out, float* d_density_p, cnb_stream_t stream);
 
 /* ---- f1 ("next" row): ray generation + AABB clipping on the device (fruit_nerf.py:283-288) ------------------------------ */
-/* nerfstudio Cameras.generate_rays for one perspective camera without distortion */
+/* nerfstudio Cameras.generate_rays for one perspective camera (without distortion; the *_lens entries add it) */
 typedef struct cnb_camera {
   float c2w[12];   /* camera-to-world [3,4], row-major (OpenGL axes: +x right, +y up, camera looks down -z) */
   float fx, fy, cx, cy;
   int32_t width, height;
 } cnb_camera;
+/* Lens distortion of an OPENCV-style perspective camera, in the order of nerfstudio's camera_utils.get_distortion_params
+ * (Cameras.distortion_params [..., 6]).  The *_lens entries undistort every normalised pixel coordinate (x, -y) -- the ray's and
+ * both pixel-area offsets -- with camera_utils.radial_and_tangential_undistort (10 Newton steps, eps 1e-3, float32 in nerfstudio's
+ * operation order) before forming the direction.  All six zero = no distortion (the solve is then the identity, bit for bit). */
+typedef struct cnb_lens {
+  float k1, k2, k3, k4, p1, p2;
+} cnb_lens;
 /* cam / aabb are HOST pointers (aabb = min xyz, max xyz; NULL = no clipping).  pixel_yx (device, optional) [n,2] integer pixel
  * rows/columns; NULL = every pixel of the image in row-major order (n = width*height).  Outputs (device): origins, directions
  * [n,3]; pixel_area [n] (optional); nears, fars [n] (with aabb: slab test, misses = 1e10 as nerfstudio's intersect_aabb);
  * valid_count (optional, device int32, ACCUMULATED) = rays that hit the box. */
 int cnb_generate_rays(const cnb_camera* cam, const int32_t* pixel_yx, int64_t n, const float* aabb, float* origins, float* directions,
                       float* pixel_area, float* nears, float* fars, int32_t* valid_count, cnb_stream_t stream);
+/* cnb_generate_rays with lens distortion: lens is a HOST pointer, NULL or all zero = cnb_generate_rays exactly. */
+int cnb_generate_rays_lens(const cnb_camera* cam, const cnb_lens* lens, const int32_t* pixel_yx, int64_t n, const float* aabb, float* origins,
+                           float* directions, float* pixel_area, float* nears, float* fars, int32_t* valid_count, cnb_stream_t stream);
 
 /* ---- e2 / e3 / f1: the loop bodies of the two export workloads around the render call -------------------------------------- */
 /* `ns-export pointcloud` (export/exporter_utils_nerfacto.py:153-176): point = origin + direction * depth; keep = (only_semantics ?
@@ -295,6 +305,11 @@ int cnb_extract_points(const float* origins, const float* directions, const floa
  * not written).  cam: HOST pointer; boxes: DEVICE [num_boxes,6] (min xyz, max xyz). */
 int cnb_generate_rays_boxes(const cnb_camera* cam, const float* boxes, int32_t num_boxes, int64_t capacity, float* origins, float* directions,
                             float* pixel_area, float* nears, float* fars, int32_t* tags, int32_t* count, cnb_stream_t stream);
+/* cnb_generate_rays_boxes with lens distortion (see cnb_lens): each pixel's ray is undistorted before the slab tests, the pixel-area
+ * offsets on its first hit.  lens: HOST pointer, NULL or all zero = cnb_generate_rays_boxes exactly. */
+int cnb_generate_rays_boxes_lens(const cnb_camera* cam, const cnb_lens* lens, const float* boxes, int32_t num_boxes, int64_t capacity,
+                                 float* origins, float* directions, float* pixel_area, float* nears, float* fars, int32_t* tags, int32_t* count,
+                                 cnb_stream_t stream);
 /* fruit_nerf.py:296-315: wo_occ[tag] = q(semantics), visible[tag] = front_opacity >= occlusion_threshold ? 0 : q(semantics), with
  * q(x) = uint8(clamp(x * 255 + 0.5, 0, 255)) (torchvision save_image); the two uint8 images [num_boxes, H*W] are cleared by the caller. */
 int cnb_projection_scatter(const int32_t* tags, const float* semantics, const float* front_opacity, int64_t n, float occlusion_threshold,
@@ -320,6 +335,11 @@ typedef struct cnb_image_set {
  * directions [R,3]; pixel_area [R] optional; camera_indices [R] int32 optional; image [R,3] and fruit_mask [R] optional. */
 int cnb_sample_train_batch(const cnb_image_set* set, const float* rand3, int64_t R, int32_t* indices, float* origins, float* directions,
                            float* pixel_area, int32_t* camera_indices, float* image, float* fruit_mask, cnb_stream_t stream);
+/* cnb_sample_train_batch with per-camera lens distortion (see cnb_lens): lenses is a DEVICE array [num_images] (zero records = no
+ * distortion for that camera) or NULL = cnb_sample_train_batch exactly. */
+int cnb_sample_train_batch_lens(const cnb_image_set* set, const cnb_lens* lenses, const float* rand3, int64_t R, int32_t* indices, float* origins,
+                                float* directions, float* pixel_area, int32_t* camera_indices, float* image, float* fruit_mask,
+                                cnb_stream_t stream);
 
 /* ---- f2: optimiser (torch.optim.Adam semantics; fruit_nerf_config.py:45-60) -------------------------------- */
 int cnb_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
