@@ -456,8 +456,9 @@ int make_args(const cnb_density_field* f, const cnb_samples* s, bool bwd, DfArgs
   }
   CNB_REQUIRE(m.dims[0] == 2 * g.num_levels, "density_field: mlp in dim %d != 2*num_levels", m.dims[0]);
   CNB_REQUIRE(m.W[0] && m.b[0] && m.W[1] && m.b[1], "density_field: null mlp weights");
-  CNB_REQUIRE(s->origins && s->directions && s->starts && s->ends, "density_field: null sample arrays");
   CNB_REQUIRE(s->samples_per_ray >= 1 && s->num_rays >= 0, "density_field: bad sample counts");
+  // an empty batch has no arrays: torch hands out null pointers for zero-size tensors
+  CNB_REQUIRE(s->num_rays == 0 || (s->origins && s->directions && s->starts && s->ends), "density_field: null sample arrays");
   CNB_REQUIRE(!bwd || g.d_table != nullptr, "density_field_bwd: d_table required");
   if (bwd)
     for (int i = 0; i < g.num_levels; ++i) CNB_REQUIRE(g.scalings[i] < 65535.0f, "density_field_bwd: level resolution %g too large for the aggregated scatter", g.scalings[i]);
@@ -527,6 +528,7 @@ int launch_bwd(const DfArgs& a, const float* d_density, cudaStream_t st) {
     if (small && H == 32) return FN<8, 32>(__VA_ARGS__);                                    \
     if (small && H == 64) return FN<8, 64>(__VA_ARGS__);                                    \
     if (!small && H == 16) return FN<16, 16>(__VA_ARGS__);                                  \
+    if (!small && H == 32) return FN<16, 32>(__VA_ARGS__);                                  \
     if (!small && H == 64) return FN<16, 64>(__VA_ARGS__);                                  \
     cnb_set_error("density_field: hidden width %d not compiled (16/32/64)", H);             \
     return CNB_ERR_UNSUPPORTED;                                                             \

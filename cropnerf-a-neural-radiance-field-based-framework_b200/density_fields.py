@@ -36,6 +36,8 @@ class HashMLPDensityField(nn.Module):
         if not use_linear:
             if num_layers != 2:
                 raise ValueError("the fused proposal kernel is compiled for num_layers=2 (nerfstudio default, fruit_nerf.py:123-139)")
+            if hidden_dim not in (16, 32, 64):
+                raise ValueError(f"the fused proposal kernel is compiled for hidden_dim 16, 32 or 64 (got {hidden_dim})")
             network = MLP(in_dim=self.encoding.get_out_dim(), num_layers=num_layers, layer_width=hidden_dim, out_dim=1,
                           activation=nn.ReLU(), out_activation=None)
             self.mlp_base = nn.Sequential(self.encoding, network)
