@@ -184,9 +184,11 @@ __device__ __forceinline__ void cnb_red4(float* table, uint32_t even_row, float 
 
 // Gradient scatter of one (sample, level) with WARP AGGREGATION.  Must be called by all 32 lanes (inactive lanes pass
 // active = false).  Lanes are consecutive samples of a ray, so samples that fall into the same grid cell form runs of
-// consecutive lanes; a run (capped at 8 lanes) is summed with a segmented warp scan and only its last lane issues the
-// reductions.  The two x-neighbours of a corner pair (hash prime of x is 1, SURVEY.md section 7) are adjacent table
-// rows whenever floor(x) is even: those go out as ONE 16-byte red.global.add.v4.f32.
+// consecutive lanes; a run (capped at CAP lanes) is summed with a segmented warp scan and only its last lane issues the
+// reductions.  The scan stops after the rounds the warp's longest run needs: a round of offset off >= that length adds
+// nothing on any lane, so the sums are those of the full log2(CAP) rounds, bit for bit, and a large cap costs shuffles
+// only in the warps whose runs are long.  The two x-neighbours of a corner pair (hash prime of x is 1, SURVEY.md
+// section 7) are adjacent table rows whenever floor(x) is even: those go out as ONE 16-byte red.global.add.v4.f32.
 // Requires integer cell coordinates < 65536 (scalings < 65535).
 template <int CAP = 8>
 __device__ __forceinline__ void cnb_scatter_cell(float* d_table, const CnbCell& c, uint32_t mask, uint32_t level_offset, float d0, float d1,
@@ -205,16 +207,17 @@ __device__ __forceinline__ void cnb_scatter_cell(float* d_table, const CnbCell& 
   float v0[8], v1[8];
 #pragma unroll
   for (int k = 0; k < 8; ++k) { v0[k] = w[k] * d0; v1[k] = w[k] * d1; }
-  if (heads != FULL) {  // at least one run of two or more lanes in this warp
-    const int start = 31 - __clz(heads & (FULL >> (31 - lane)));
+  // lane 0 is always a head, so every lane has a run start; depth + 1 is the warp's longest run (warp-uniform)
+  const int start = 31 - __clz(heads & (FULL >> (31 - lane)));
+  const int depth = (int)__reduce_max_sync(FULL, (unsigned)(lane - start));
 #pragma unroll
-    for (int off = 1; off < CAP; off <<= 1) {
-      const bool take = lane - off >= start;
+  for (int off = 1; off < CAP; off <<= 1) {
+    if (off > depth) break;
+    const bool take = lane - off >= start;
 #pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        const float t0 = __shfl_up_sync(FULL, v0[k], off), t1 = __shfl_up_sync(FULL, v1[k], off);
-        if (take) { v0[k] += t0; v1[k] += t1; }
-      }
+    for (int k = 0; k < 8; ++k) {
+      const float t0 = __shfl_up_sync(FULL, v0[k], off), t1 = __shfl_up_sync(FULL, v1[k], off);
+      if (take) { v0[k] += t0; v1[k] += t1; }
     }
   }
   const bool tail = lane == 31 || ((heads >> (lane + 1)) & 1u);
