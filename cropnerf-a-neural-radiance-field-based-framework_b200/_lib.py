@@ -146,6 +146,7 @@ class Model(C.Structure):
         ("bg_mode", C.c_int32),
         ("bg_color", C.c_float * 3),
         ("ray_gradients", C.c_int32),
+        ("field_table_half", C.c_void_p),
     ]
 
 
@@ -168,6 +169,11 @@ class OptGroup(C.Structure):
     _fields_ = [("param", C.c_void_p), ("grad", C.c_void_p), ("exp_avg", C.c_void_p), ("exp_avg_sq", C.c_void_p), ("n", C.c_int64), ("scalars", C.c_void_p),
                 ("chain", C.c_int32), ("_pad", C.c_int32), ("live", C.c_void_p), ("peer_comm", C.c_void_p), ("peer_group", C.c_void_p),
                 ("peer_flags", C.c_int32), ("peer_channel", C.c_int32)]
+
+
+class OptHalf(C.Structure):
+    """cnb_opt_half: the fp16 copy of a hash table inside an optimiser group."""
+    _fields_ = [("table_half", C.c_void_p), ("first", C.c_int64), ("count", C.c_int64)]
 
 
 class TrainCfg(C.Structure):
@@ -193,6 +199,7 @@ class TrainCfg(C.Structure):
         ("trans_l2_penalty", C.c_float),
         ("rot_l2_penalty", C.c_float),
         ("_pad_camopt", C.c_int32),
+        ("opt_half", OptHalf * MAX_OPT_GROUPS),
     ]
 
 
@@ -227,6 +234,8 @@ SIGNATURES = {
     "cnb_device_count": (C.c_int, []),
     "cnb_hashgrid_fwd": (C.c_int, [C.POINTER(Grid), _P, _I64, _P, _P, _P]),
     "cnb_hashgrid_bwd": (C.c_int, [C.POINTER(Grid), _P, _P, _I64, _P]),
+    "cnb_hashgrid_fwd_half": (C.c_int, [C.POINTER(Grid), _P, _P, _I64, _P, _P, _P]),
+    "cnb_table_to_half": (C.c_int, [_P, _I64, _P, _I64, _P, _P]),
     "cnb_mlp_hidden_floats": (_I64, [C.POINTER(Mlp)]),
     "cnb_mlp_fwd": (C.c_int, [C.POINTER(Mlp), _P, _I64, _I64, _P, _P, _P]),
     "cnb_mlp_bwd": (C.c_int, [C.POINTER(Mlp), _P, _I64, _P, _P, _P, _I64, _P, _I64, _P]),
@@ -238,12 +247,15 @@ SIGNATURES = {
     "cnb_field_ctx_floats": (_I64, [C.POINTER(Field), _I64, _I32]),
     "cnb_field_fwd": (C.c_int, [C.POINTER(Field), C.POINTER(Samples), _P, _P, _P, _P, _P, _P, _I32, _P]),
     "cnb_field_bwd": (C.c_int, [C.POINTER(Field), C.POINTER(Samples), _P, _P, _P, _P, _P, _P]),
+    "cnb_field_fwd_half": (C.c_int, [C.POINTER(Field), _P, C.POINTER(Samples), _P, _P, _P, _P, _P, _P, _I32, _P]),
     "cnb_density_field_fwd_keep": (C.c_int, [C.POINTER(DensityField), C.POINTER(Samples), _P, _P, _P]),
     "cnb_density_field_bwd_kept": (C.c_int, [C.POINTER(DensityField), C.POINTER(Samples), _P, _P, _P]),
     "cnb_density_field_kept_supported": (C.c_int, [C.POINTER(DensityField)]),
     "cnb_position_grad_rays": (C.c_int, [C.POINTER(Grid), C.POINTER(Warp), C.POINTER(Samples), _P, _P, _P, _P]),
     "cnb_density_field_bwd_rays": (C.c_int, [C.POINTER(DensityField), C.POINTER(Samples), _P, _P, _P, _P, _P]),
     "cnb_field_bwd_rays": (C.c_int, [C.POINTER(Field), C.POINTER(Samples), _P, _P, _P, _P, _P, _P, _P, _P]),
+    "cnb_position_grad_rays_half": (C.c_int, [C.POINTER(Grid), _P, C.POINTER(Warp), C.POINTER(Samples), _P, _P, _P, _P]),
+    "cnb_field_bwd_rays_half": (C.c_int, [C.POINTER(Field), _P, C.POINTER(Samples), _P, _P, _P, _P, _P, _P, _P, _P]),
     "cnb_generate_rays": (C.c_int, [C.POINTER(Camera), _P, _I64, C.POINTER(_F), _P, _P, _P, _P, _P, _P, _P]),
     "cnb_generate_rays_lens": (C.c_int, [C.POINTER(Camera), C.POINTER(Lens), _P, _I64, C.POINTER(_F), _P, _P, _P, _P, _P, _P, _P]),
     "cnb_camera_opt_apply": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P, _P, _P]),
@@ -278,6 +290,8 @@ SIGNATURES = {
     "cnb_upload": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int64), _I32, _P]),
     "cnb_stage_inputs": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int64), _I32, _P, C.POINTER(_F), _I32, _P]),
     "cnb_adam_step_zero_dev": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P]),
+    "cnb_adam_step_zero_half": (C.c_int, [_P, _P, _P, _P, _I64, _F, _F, _F, _F, _I32, _F, _P, _P, _P, _I64, _I64, _P]),
+    "cnb_adam_step_zero_dev_half": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _P, _I64, _I64, _P]),
     "cnb_p2p_owned_range": (None, [_I64, _I32, _I32, C.POINTER(_I64), C.POINTER(_I64)]),
     "cnb_p2p_barrier": (C.c_int, [C.POINTER(P2PComm), _P]),
     "cnb_ddp_exchange_dev": (C.c_int, [C.POINTER(P2PComm), C.POINTER(P2PGroup), _P, _P, _P, _I64, _P, _I32, _I32, _P]),

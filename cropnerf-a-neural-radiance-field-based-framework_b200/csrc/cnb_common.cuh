@@ -4,6 +4,7 @@
 // round-to-nearest intrinsics (__fmul_rn/__fadd_rn/__fdiv_rn) so nvcc cannot contract it into FMAs; the
 // torch reference evaluates each elementwise op as a separately rounded fp32 operation.
 #pragma once
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -149,6 +150,10 @@ __device__ __forceinline__ float2 cnb_ldg2(const float* table, uint32_t row) {
   return __ldg(reinterpret_cast<const float2*>(table) + row);
 }
 
+// fp16 copy of a table (one __half2 per row): the row widened to fp32 exactly, so a blend of these values is the fp32 blend of a table holding
+// table.half().float()
+__device__ __forceinline__ float2 cnb_ldg2(const __half2* table, uint32_t row) { return __half22float2(__ldg(table + row)); }
+
 // The 8 corner rows of a cell.  The hash prime of x is 1, so the ceil-x / floor-x rows of a corner pair differ only in
 // bit 0 whenever floor(x) is even: those pairs -- (0,3) (1,2) (5,6) (4,7) in the reference's corner order -- are fetched
 // with ONE 16-byte load.  The gathers are bound by the L1TEX data pipe (one wavefront per distinct sector per request),
@@ -165,6 +170,24 @@ __device__ __forceinline__ void cnb_gather8(const float* __restrict__ table, con
       const bool f_even = (h[pf[q]] & 1u) == 0u;
       v[pf[q]] = f_even ? make_float2(w.x, w.y) : make_float2(w.z, w.w);
       v[pc[q]] = f_even ? make_float2(w.z, w.w) : make_float2(w.x, w.y);
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) v[k] = cnb_ldg2(table, h[k]);
+  }
+}
+
+// cnb_gather8 on an fp16 copy of the table: the x-neighbour pair of a corner (adjacent rows when floor(x) is even) is ONE 8-byte load.
+__device__ __forceinline__ void cnb_gather8(const __half2* __restrict__ table, const CnbCell& c, const uint32_t (&h)[8], float2 (&v)[8]) {
+  if (c.cx == c.fx + 1u && (c.fx & 1u) == 0u) {
+    const int pc[4] = {0, 1, 5, 4}, pf[4] = {3, 2, 6, 7};
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const uint2 w = __ldg(reinterpret_cast<const uint2*>(table) + (h[pf[q]] >> 1));
+      const float2 lo = __half22float2(*reinterpret_cast<const __half2*>(&w.x)), hi = __half22float2(*reinterpret_cast<const __half2*>(&w.y));
+      const bool f_even = (h[pf[q]] & 1u) == 0u;
+      v[pf[q]] = f_even ? lo : hi;
+      v[pc[q]] = f_even ? hi : lo;
     }
   } else {
 #pragma unroll

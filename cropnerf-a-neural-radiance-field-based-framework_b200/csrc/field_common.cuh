@@ -28,6 +28,8 @@ __device__ __forceinline__ void cnb_sh16(float dx, float dy, float dz, float (&c
 }
 
 int cnb_field_check(const cnb_field* f, const cnb_samples* s, bool bwd);
+// CNB_OK when table_half is NULL or the field runs on the layer-by-layer mixed path, else CNB_ERR_UNSUPPORTED with the reason (field_fp32.cu)
+int cnb_field_check_half(const cnb_field* f, const void* table_half);
 
 // mixed-precision (tensor-core) implementation: field_mixed.cu, the backward in field_mixed_bwd_tc5.cu
 int cnb_field_mixed_fwd(const cnb_field* f, const cnb_samples* s, float* density, float* geo, float* rgb, float* sem, float* positions_out, float* ctx,

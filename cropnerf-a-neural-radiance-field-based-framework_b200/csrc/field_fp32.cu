@@ -198,10 +198,26 @@ extern "C" int64_t cnb_field_ctx_floats(const cnb_field* f, int64_t n, int32_t t
   return make_layout(f, n, training != 0).total;
 }
 
+// fp16 tables are compiled for the layer-by-layer mixed path only: the fused base kernels' 64 MiB table sits in L2, where 4-byte rows gather no
+// faster than 8-byte ones (DESIGN.md section 7)
+int cnb_field_check_half(const cnb_field* f, const void* table_half) {
+  if (table_half == nullptr || mixed_wide(f)) return CNB_OK;
+  cnb_set_error(f->precision != CNB_PREC_MIXED ? "field: fp16 tables are compiled for precision=mixed only (exact fp32 mode keeps the fp32 table)"
+                                               : "field: fp16 tables are compiled for the layer-by-layer mixed path (big / huge presets) only: the fused "
+                                                 "base-preset kernels read a table that fits L2, where fp16 rows gather no faster");
+  return CNB_ERR_UNSUPPORTED;
+}
+
 extern "C" int cnb_field_fwd(const cnb_field* f, const cnb_samples* s, float* density, float* geo, float* rgb, float* sem, float* positions_out,
                              float* ctx, int32_t training, cnb_stream_t stream) {
+  return cnb_field_fwd_half(f, nullptr, s, density, geo, rgb, sem, positions_out, ctx, training, stream);
+}
+
+extern "C" int cnb_field_fwd_half(const cnb_field* f, const void* table_half, const cnb_samples* s, float* density, float* geo, float* rgb, float* sem,
+                                  float* positions_out, float* ctx, int32_t training, cnb_stream_t stream) {
   int rc = cnb_field_check(f, s, false);
   if (rc) return rc;
+  if ((rc = cnb_field_check_half(f, table_half))) return rc;
   const int64_t N = s->num_rays * s->samples_per_ray;
   if (N == 0) return CNB_OK;
   CNB_REQUIRE(density != nullptr, "field_fwd: null density output");
@@ -227,7 +243,7 @@ extern "C" int cnb_field_fwd(const cnb_field* f, const cnb_samples* s, float* de
   float* pos = ctx + c.pos; float* sel = ctx + c.sel; float* x0 = ctx + c.x0; float* bo = ctx + c.bo;
   k_positions<<<grid1d(N, 256), 256, 0, stream>>>(*s, f->warp, pos, sel, positions_out);
   if ((rc = cnb_check_launch("field positions"))) return rc;
-  if ((rc = cnb_hashgrid_fwd(&f->grid, pos, N, x0, nullptr, stream))) return rc;
+  if ((rc = cnb_hashgrid_fwd_half(&f->grid, table_half, pos, N, x0, nullptr, stream))) return rc;
   if ((rc = mlp_fwd(&f->base, x0, c.in0, bo, c.hb))) return rc;
   k_mid_fwd<<<grid1d(N, 256), 256, 0, stream>>>(*s, bo, c.ob, sel, f->embedding, f->mean_embedding, f->appearance_mode, f->appearance_dim, c.rip, density,
                                                  geo, ctx + c.rin);
@@ -301,8 +317,15 @@ extern "C" int cnb_field_bwd(const cnb_field* f, const cnb_samples* s, const flo
 // d(features) row-major.
 extern "C" int cnb_field_bwd_rays(const cnb_field* f, const cnb_samples* s, const float* d_density, const float* d_rgb, const float* d_sem,
                                   const float* d_geo, float* ctx, float* d_origins, float* d_directions, cnb_stream_t stream) {
+  return cnb_field_bwd_rays_half(f, nullptr, s, d_density, d_rgb, d_sem, d_geo, ctx, d_origins, d_directions, stream);
+}
+
+extern "C" int cnb_field_bwd_rays_half(const cnb_field* f, const void* table_half, const cnb_samples* s, const float* d_density, const float* d_rgb,
+                                       const float* d_sem, const float* d_geo, float* ctx, float* d_origins, float* d_directions, cnb_stream_t stream) {
   CNB_REQUIRE(d_origins && d_directions, "field_bwd_rays: null ray gradients");
-  int rc = cnb_field_bwd(f, s, d_density, d_rgb, d_sem, d_geo, ctx, stream);
+  int rc = cnb_field_check_half(f, table_half);
+  if (rc) return rc;
+  rc = cnb_field_bwd(f, s, d_density, d_rgb, d_sem, d_geo, ctx, stream);
   if (rc) return rc;
   const int64_t N = s->num_rays * s->samples_per_ray;
   if (N == 0) return CNB_OK;
@@ -311,5 +334,5 @@ extern "C" int cnb_field_bwd_rays(const cnb_field* f, const cnb_samples* s, cons
     CNB_REQUIRE(f->grid.num_levels == 16, "field_bwd_rays: the mixed path stores d(features) as [16][N][2]; num_levels must be 16");
     return cnb_position_grad_rays_level_major(&f->grid, &f->warp, s, cnb_field_mixed_dx0(ctx, N), d_origins, d_directions, stream);
   }
-  return cnb_position_grad_rays(&f->grid, &f->warp, s, ctx + make_layout(f, N, true, wide).d_x0, d_origins, d_directions, stream);
+  return cnb_position_grad_rays_half(&f->grid, table_half, &f->warp, s, ctx + make_layout(f, N, true, wide).d_x0, d_origins, d_directions, stream);
 }

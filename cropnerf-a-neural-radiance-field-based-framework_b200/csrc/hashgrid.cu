@@ -4,22 +4,29 @@
 //
 // One thread per (sample, level): 8 independent 8-byte gathers in flight per thread, coalesced 8-byte
 // stores of the [n, 2L] feature rows.  HBM/L2-bound: 8 corners * 8 B per (sample, level).
+#include <type_traits>
+
 #include "cnb_common.cuh"
 
 namespace {
 
-struct GridArgs {
-  const float* table;
+// Row = float: the fp32 table (two floats per row); Row = __half2: its fp16 copy (cnb_table_to_half), same layout otherwise
+template <typename Row>
+struct GridArgsT {
+  const Row* table;
   float* d_table;
   int32_t L;
   uint32_t mask;
   uint32_t T;
   float scalings[CNB_MAX_LEVELS];
 };
+using GridArgs = GridArgsT<float>;
 
-GridArgs make_args(const cnb_grid* g) {
-  GridArgs a;
-  a.table = g->table;
+template <typename Row = float>
+GridArgsT<Row> make_args(const cnb_grid* g, const Row* table = nullptr) {
+  GridArgsT<Row> a;
+  a.table = table;
+  if constexpr (std::is_same<Row, float>::value) a.table = g->table;
   a.d_table = g->d_table;
   a.L = g->num_levels;
   a.T = 1u << g->log2_hashmap_size;
@@ -30,7 +37,9 @@ GridArgs make_args(const cnb_grid* g) {
 
 // Forward: a warp owns 32 CONSECUTIVE samples of one level, so one load instruction touches few distinct 128-byte lines at
 // the coarse / middle levels (the gathers are bound by the L1TEX t-stage: one wavefront per distinct line per request).
-__global__ void __launch_bounds__(256) k_hashgrid_fwd(const __grid_constant__ GridArgs g, const float* __restrict__ pos, int64_t n, float* __restrict__ out,
+// The fp16 rows are gathered with cnb_gather8 (x-neighbour pairs as one 8-byte load); the fp32 rows keep eight 8-byte loads.
+template <typename Row>
+__global__ void __launch_bounds__(256) k_hashgrid_fwd(const __grid_constant__ GridArgsT<Row> g, const float* __restrict__ pos, int64_t n, float* __restrict__ out,
                                                        int32_t* __restrict__ indices) {
   const int lane = threadIdx.x & 31;
   const int64_t nblk = (n + 31) >> 5;
@@ -47,8 +56,12 @@ __global__ void __launch_bounds__(256) k_hashgrid_fwd(const __grid_constant__ Gr
     uint32_t h[8];
     cnb_corner_rows(c, g.mask, (uint32_t)l * g.T, h);
     float2 v[8];
+    if constexpr (std::is_same<Row, float>::value) {
 #pragma unroll
-    for (int k = 0; k < 8; ++k) v[k] = cnb_ldg2(g.table, h[k]);
+      for (int k = 0; k < 8; ++k) v[k] = cnb_ldg2(g.table, h[k]);
+    } else {
+      cnb_gather8(g.table, c, h, v);
+    }
     float f0[8], f1[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) { f0[k] = v[k].x; f1[k] = v[k].y; }
@@ -98,8 +111,8 @@ __global__ void __launch_bounds__(256) k_hashgrid_bwd(const __grid_constant__ Gr
 //   * applies the selector mask, the (c+2)/4 or AABB normalisation and the Jacobian of SceneContraction(order=inf),
 //   * reduces dL/dp over the ray (d_origins += dL/dp, d_directions += (s+e)/2 * dL/dp): warp shuffle when the 32 lanes
 //     share the ray, atomics otherwise.
-template <bool LM>  // LM: d_feat is level-major [L][total][2]
-__global__ void __launch_bounds__(128) k_position_grad_rays(const __grid_constant__ GridArgs g, cnb_warp wp, cnb_samples sm, const float* __restrict__ d_feat,
+template <bool LM, typename Row = float>  // LM: d_feat is level-major [L][total][2]; Row: the rows the forward gathered
+__global__ void __launch_bounds__(128) k_position_grad_rays(const __grid_constant__ GridArgsT<Row> g, cnb_warp wp, cnb_samples sm, const float* __restrict__ d_feat,
                                                             float* __restrict__ d_origins, float* __restrict__ d_directions) {
   const int S = sm.samples_per_ray;
   const int64_t total = sm.num_rays * S;
@@ -206,12 +219,22 @@ static int check_grid(const cnb_grid* g, bool need_grad) {
 }
 
 extern "C" int cnb_hashgrid_fwd(const cnb_grid* g, const float* positions, int64_t n, float* out, int32_t* indices, cnb_stream_t stream) {
+  return cnb_hashgrid_fwd_half(g, nullptr, positions, n, out, indices, stream);
+}
+
+extern "C" int cnb_hashgrid_fwd_half(const cnb_grid* g, const void* table_half, const float* positions, int64_t n, float* out, int32_t* indices,
+                                     cnb_stream_t stream) {
   int rc = check_grid(g, false);
   if (rc) return rc;
   CNB_REQUIRE(n >= 0 && (n == 0 || (positions && out)), "hashgrid_fwd: null positions/out");
   if (n == 0) return CNB_OK;
-  GridArgs a = make_args(g);
-  k_hashgrid_fwd<<<grid_for(((n + 31) / 32) * 32 * a.L, 256), 256, 0, stream>>>(a, positions, n, out, indices);
+  const int blocks = grid_for(((n + 31) / 32) * 32 * g->num_levels, 256);
+  if (table_half != nullptr) {
+    CNB_REQUIRE(((uintptr_t)table_half & 7) == 0, "hashgrid_fwd: the fp16 table must be 8-byte aligned");
+    k_hashgrid_fwd<__half2><<<blocks, 256, 0, stream>>>(make_args(g, static_cast<const __half2*>(table_half)), positions, n, out, indices);
+  } else {
+    k_hashgrid_fwd<float><<<blocks, 256, 0, stream>>>(make_args(g), positions, n, out, indices);
+  }
   return cnb_check_launch("hashgrid_fwd");
 }
 
@@ -237,29 +260,40 @@ int cnb_hashgrid_bwd_level_major(const cnb_grid* g, const float* positions, cons
   return hashgrid_bwd_impl(g, positions, d_out, n, true, stream);
 }
 
-static int position_grad_rays_impl(const cnb_grid* g, const cnb_warp* warp, const cnb_samples* s, const float* d_feat, float* d_origins,
-                                   float* d_directions, bool level_major, cnb_stream_t stream) {
+static int position_grad_rays_impl(const cnb_grid* g, const __half2* table_half, const cnb_warp* warp, const cnb_samples* s, const float* d_feat,
+                                   float* d_origins, float* d_directions, bool level_major, cnb_stream_t stream) {
   int rc = check_grid(g, false);
   if (rc) return rc;
   CNB_REQUIRE(warp && s && d_feat && d_origins && d_directions, "position_grad_rays: null pointer");
   CNB_REQUIRE(s->origins && s->directions && s->starts && s->ends && s->samples_per_ray >= 1 && s->num_rays >= 0, "position_grad_rays: bad samples");
   const int64_t total = s->num_rays * s->samples_per_ray;
   if (total == 0) return CNB_OK;
+  const int blocks = grid_for(total, 128);
+  if (table_half != nullptr) {
+    CNB_REQUIRE(!level_major, "position_grad_rays: the fp16 table is read by the layer-by-layer field path only");
+    k_position_grad_rays<false, __half2><<<blocks, 128, 0, stream>>>(make_args(g, table_half), *warp, *s, d_feat, d_origins, d_directions);
+    return cnb_check_launch("position_grad_rays");
+  }
   GridArgs a = make_args(g);
-  if (level_major) k_position_grad_rays<true><<<grid_for(total, 128), 128, 0, stream>>>(a, *warp, *s, d_feat, d_origins, d_directions);
-  else k_position_grad_rays<false><<<grid_for(total, 128), 128, 0, stream>>>(a, *warp, *s, d_feat, d_origins, d_directions);
+  if (level_major) k_position_grad_rays<true><<<blocks, 128, 0, stream>>>(a, *warp, *s, d_feat, d_origins, d_directions);
+  else k_position_grad_rays<false><<<blocks, 128, 0, stream>>>(a, *warp, *s, d_feat, d_origins, d_directions);
   return cnb_check_launch("position_grad_rays");
 }
 
 extern "C" int cnb_position_grad_rays(const cnb_grid* g, const cnb_warp* warp, const cnb_samples* s, const float* d_feat, float* d_origins,
                                       float* d_directions, cnb_stream_t stream) {
-  return position_grad_rays_impl(g, warp, s, d_feat, d_origins, d_directions, false, stream);
+  return position_grad_rays_impl(g, nullptr, warp, s, d_feat, d_origins, d_directions, false, stream);
+}
+
+extern "C" int cnb_position_grad_rays_half(const cnb_grid* g, const void* table_half, const cnb_warp* warp, const cnb_samples* s, const float* d_feat,
+                                           float* d_origins, float* d_directions, cnb_stream_t stream) {
+  return position_grad_rays_impl(g, static_cast<const __half2*>(table_half), warp, s, d_feat, d_origins, d_directions, false, stream);
 }
 
 // library-internal: d_feat level-major [L][total][2]
 int cnb_position_grad_rays_level_major(const cnb_grid* g, const cnb_warp* warp, const cnb_samples* s, const float* d_feat, float* d_origins,
                                        float* d_directions, cudaStream_t stream) {
-  return position_grad_rays_impl(g, warp, s, d_feat, d_origins, d_directions, true, stream);
+  return position_grad_rays_impl(g, nullptr, warp, s, d_feat, d_origins, d_directions, true, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -318,4 +352,35 @@ extern "C" int cnb_bitmap_mark_range(uint32_t* bitmap, int64_t first_unit, int64
   if (blocks > cap) blocks = cap;
   k_mark_range<<<(int)blocks, 256, 0, stream>>>(bitmap, first_unit, units);
   return cnb_check_launch("bitmap_mark_range");
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// fp16 copy of a table (initialisation, checkpoint load, writes made outside the optimiser): dst[i] = __float2half_rn(src[i]).  With `live`, only
+// the 16-byte units whose bit (first_unit + i / 4) is set are written -- the rows the optimiser updates; the others keep what they hold.
+namespace {
+__global__ void __launch_bounds__(256) k_table_to_half(const float4* __restrict__ src, int64_t n4, const uint32_t* __restrict__ live, int64_t first_unit,
+                                                       uint2* __restrict__ dst) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+    if (live != nullptr) {
+      const int64_t u = first_unit + i;
+      if (!((__ldg(live + (u >> 5)) >> (u & 31)) & 1u)) continue;
+    }
+    const float4 v = __ldg(src + i);
+    const __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
+    dst[i] = make_uint2(*reinterpret_cast<const uint32_t*>(&a), *reinterpret_cast<const uint32_t*>(&b));
+  }
+}
+}  // namespace
+
+extern "C" int cnb_table_to_half(const float* table, int64_t n, const uint32_t* live, int64_t first_unit, void* table_half, cnb_stream_t stream) {
+  CNB_REQUIRE(n >= 0 && n % 4 == 0 && first_unit >= 0, "table_to_half: n = %lld must be a multiple of 4", (long long)n);
+  if (n == 0) return CNB_OK;
+  CNB_REQUIRE(table && table_half, "table_to_half: null pointer");
+  CNB_REQUIRE((((uintptr_t)table & 15) | ((uintptr_t)table_half & 7)) == 0, "table_to_half: table must be 16-byte, table_half 8-byte aligned");
+  const int64_t n4 = n / 4;
+  int64_t blocks = (n4 + 255) / 256;
+  const int64_t cap = (int64_t)cnb_num_sms() * 16;
+  if (blocks > cap) blocks = cap;
+  k_table_to_half<<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<const float4*>(table), n4, live, first_unit, static_cast<uint2*>(table_half));
+  return cnb_check_launch("table_to_half");
 }

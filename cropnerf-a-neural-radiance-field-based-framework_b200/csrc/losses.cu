@@ -140,9 +140,28 @@ __global__ void __launch_bounds__(256) k_adam(float* __restrict__ p, const float
 // hoists the (independent) zero store right behind the loads, and a store to a line whose load is still in flight
 // serialises the LSU -- the pass then runs at 2.0 TB/s instead of 6.3 TB/s on B200 (tests/micro/adam_bench.cu:
 // a_current vs f_late_zero; store cache policy makes no difference).
+// HALF: the group holds a hash table with an fp16 copy (cnb_table_to_half); every updated float4 of the table's range [first4, first4 + count4)
+// is also stored rounded to fp16 (8 bytes, from registers).  Units the update skips (unreachable rows, a skipped step) keep their copy.
+struct HalfDst {
+  uint2* dst;
+  int64_t first4, count4;
+};
+
+template <bool HALF>
+__device__ __forceinline__ void store_half(const HalfDst& hd, int64_t i, const float4& p) {
+  if constexpr (HALF) {
+    const int64_t j = i - hd.first4;
+    if (j >= 0 && j < hd.count4) {
+      const __half2 a = __floats2half2_rn(p.x, p.y), b = __floats2half2_rn(p.z, p.w);
+      hd.dst[j] = make_uint2(*reinterpret_cast<const uint32_t*>(&a), *reinterpret_cast<const uint32_t*>(&b));
+    }
+  }
+}
+
+template <bool HALF>
 __global__ void __launch_bounds__(256) k_adam_zero4(float4* __restrict__ p, float4* __restrict__ g, float4* __restrict__ m, float4* __restrict__ v,
                                                     int64_t n4, float lr, float b1, float b2, float eps, float bc1, float bc2_sqrt, float inv_scale,
-                                                    const int32_t* __restrict__ skip, const uint32_t* __restrict__ live) {
+                                                    const int32_t* __restrict__ skip, const uint32_t* __restrict__ live, const HalfDst hd) {
   const float step_size = lr / bc1;
   if (skip != nullptr && __ldg(skip) != 0) {
     // GradScaler.step: a non-finite gradient was found -> the optimizer step is skipped, the gradient is still cleared
@@ -164,13 +183,15 @@ __global__ void __launch_bounds__(256) k_adam_zero4(float4* __restrict__ p, floa
     float z;
     asm volatile("mov.f32 %0, 0f00000000;" : "=f"(z) : "f"(pi.w));  // zero that "depends" on the finished update
     m[i] = mi; v[i] = vi; p[i] = pi;
+    store_half<HALF>(hd, i, pi);
     g[i] = make_float4(z, z, z, z);
   }
 }
 
 // k_adam_zero4 with the step's scalars in device memory (read once per thread through the constant-like path)
+template <bool HALF>
 __global__ void __launch_bounds__(256) k_adam_zero4_dev(float4* __restrict__ p, float4* __restrict__ g, float4* __restrict__ m, float4* __restrict__ v,
-                                                        int64_t n4, const float* __restrict__ sc, const uint32_t* __restrict__ live) {
+                                                        int64_t n4, const float* __restrict__ sc, const uint32_t* __restrict__ live, const HalfDst hd) {
   const float lr = __ldg(sc), b1 = __ldg(sc + 1), b2 = __ldg(sc + 2), eps = __ldg(sc + 3), bc1 = __ldg(sc + 4), bc2_sqrt = __ldg(sc + 5), inv_scale = __ldg(sc + 6);
   const float step_size = lr / bc1;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
@@ -187,6 +208,7 @@ __global__ void __launch_bounds__(256) k_adam_zero4_dev(float4* __restrict__ p, 
     float z;
     asm volatile("mov.f32 %0, 0f00000000;" : "=f"(z) : "f"(pi.w));  // see k_adam_zero4: the clear is issued last
     m[i] = mi; v[i] = vi; p[i] = pi;
+    store_half<HALF>(hd, i, pi);
     g[i] = make_float4(z, z, z, z);
   }
 }
@@ -286,8 +308,36 @@ extern "C" int cnb_adam_step_zero_dev_live(float* param, float* grad, float* exp
 extern "C" int cnb_adam_step_zero_dev(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, const float* scalars, cnb_stream_t stream) {
   return cnb_adam_step_zero_dev_live(param, grad, exp_avg, exp_avg_sq, n, scalars, nullptr, stream);
 }
+// the fp16 copy of a table inside a flat group: float range [first, first + count) of the group, both multiples of 4
+static int half_dst(void* table_half, int64_t first, int64_t count, int64_t n, HalfDst& hd) {
+  hd.dst = static_cast<uint2*>(table_half);
+  hd.first4 = first / 4;
+  hd.count4 = count / 4;
+  CNB_REQUIRE(table_half != nullptr && ((uintptr_t)table_half & 7) == 0, "adam: the fp16 table copy must be a non-null 8-byte aligned pointer");
+  CNB_REQUIRE(first >= 0 && count >= 0 && first % 4 == 0 && count % 4 == 0 && first + count <= n,
+              "adam: fp16 table range [%lld, %lld) must lie inside the group (%lld floats) on 4-float boundaries", (long long)first,
+              (long long)(first + count), (long long)n);
+  return CNB_OK;
+}
+
+static int adam_dev_impl(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, const float* scalars, const uint32_t* live,
+                         const HalfDst* hd, cnb_stream_t stream);
+
 extern "C" int cnb_adam_step_zero_dev_live(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, const float* scalars, const uint32_t* live,
                                            cnb_stream_t stream) {
+  return adam_dev_impl(param, grad, exp_avg, exp_avg_sq, n, scalars, live, nullptr, stream);
+}
+
+extern "C" int cnb_adam_step_zero_dev_half(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, const float* scalars,
+                                           const uint32_t* live, void* table_half, int64_t half_first, int64_t half_count, cnb_stream_t stream) {
+  HalfDst hd;
+  int rc = half_dst(table_half, half_first, half_count, n, hd);
+  if (rc) return rc;
+  return adam_dev_impl(param, grad, exp_avg, exp_avg_sq, n, scalars, live, &hd, stream);
+}
+
+static int adam_dev_impl(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, const float* scalars, const uint32_t* live,
+                         const HalfDst* hd, cnb_stream_t stream) {
   CNB_REQUIRE(n >= 0, "adam_dev: bad n");
   if (n == 0) return CNB_OK;
   CNB_REQUIRE(param && grad && exp_avg && exp_avg_sq && scalars, "adam_dev: null pointer");
@@ -297,8 +347,12 @@ extern "C" int cnb_adam_step_zero_dev_live(float* param, float* grad, float* exp
   int64_t blocks = (n4 + 255) / 256;
   const int64_t cap = (int64_t)cnb_num_sms() * 16;
   if (blocks > cap) blocks = cap;
-  k_adam_zero4_dev<<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<float4*>(param), reinterpret_cast<float4*>(grad), reinterpret_cast<float4*>(exp_avg),
-                                                    reinterpret_cast<float4*>(exp_avg_sq), n4, scalars, live);
+  if (hd != nullptr)
+    k_adam_zero4_dev<true><<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<float4*>(param), reinterpret_cast<float4*>(grad),
+                                                            reinterpret_cast<float4*>(exp_avg), reinterpret_cast<float4*>(exp_avg_sq), n4, scalars, live, *hd);
+  else
+    k_adam_zero4_dev<false><<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<float4*>(param), reinterpret_cast<float4*>(grad),
+                                                             reinterpret_cast<float4*>(exp_avg), reinterpret_cast<float4*>(exp_avg_sq), n4, scalars, live, HalfDst{});
   return cnb_check_launch("adam_zero_dev");
 }
 
@@ -317,7 +371,19 @@ extern "C" int cnb_grad_check_finite(const float* grad, int64_t n, int32_t* foun
 }
 
 static int adam_step_zero_impl(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1, float beta2,
-                               float eps, int32_t step, float inv_grad_scale, const int32_t* skip_flag, cnb_stream_t stream, const uint32_t* live = nullptr);
+                               float eps, int32_t step, float inv_grad_scale, const int32_t* skip_flag, cnb_stream_t stream, const uint32_t* live = nullptr,
+                               const HalfDst* hd = nullptr);
+
+extern "C" int cnb_adam_step_zero_half(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1, float beta2,
+                                       float eps, int32_t step, float inv_grad_scale, const int32_t* skip_flag, const uint32_t* live, void* table_half,
+                                       int64_t half_first, int64_t half_count, cnb_stream_t stream) {
+  CNB_REQUIRE(n % 4 == 0 && ((((uintptr_t)param | (uintptr_t)grad | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) & 15) == 0),
+              "adam_step_zero_half: needs a 16-byte aligned flat group with n % 4 == 0");
+  HalfDst hd;
+  int rc = half_dst(table_half, half_first, half_count, n, hd);
+  if (rc) return rc;
+  return adam_step_zero_impl(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, step, inv_grad_scale, skip_flag, stream, live, &hd);
+}
 
 extern "C" int cnb_adam_step_zero_live(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1, float beta2,
                                        float eps, int32_t step, float inv_grad_scale, const uint32_t* live, cnb_stream_t stream) {
@@ -339,7 +405,8 @@ extern "C" int cnb_adam_step_zero_guarded(float* param, float* grad, float* exp_
 }
 
 static int adam_step_zero_impl(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1, float beta2,
-                               float eps, int32_t step, float inv_grad_scale, const int32_t* skip_flag, cnb_stream_t stream, const uint32_t* live) {
+                               float eps, int32_t step, float inv_grad_scale, const int32_t* skip_flag, cnb_stream_t stream, const uint32_t* live,
+                               const HalfDst* hd) {
   CNB_REQUIRE(n >= 0 && step >= 1, "adam: bad n/step");
   if (n == 0) return CNB_OK;
   CNB_REQUIRE(param && grad && exp_avg && exp_avg_sq, "adam: null pointer");
@@ -356,7 +423,13 @@ static int adam_step_zero_impl(float* param, float* grad, float* exp_avg, float*
   int64_t blocks = (n4 + 255) / 256;
   const int64_t cap = (int64_t)cnb_num_sms() * 16;
   if (blocks > cap) blocks = cap;
-  k_adam_zero4<<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<float4*>(param), reinterpret_cast<float4*>(grad), reinterpret_cast<float4*>(exp_avg),
-                                                reinterpret_cast<float4*>(exp_avg_sq), n4, lr, beta1, beta2, eps, (float)bc1, (float)sqrt(bc2), inv_grad_scale, skip_flag, live);
+  if (hd != nullptr)
+    k_adam_zero4<true><<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<float4*>(param), reinterpret_cast<float4*>(grad), reinterpret_cast<float4*>(exp_avg),
+                                                        reinterpret_cast<float4*>(exp_avg_sq), n4, lr, beta1, beta2, eps, (float)bc1, (float)sqrt(bc2),
+                                                        inv_grad_scale, skip_flag, live, *hd);
+  else
+    k_adam_zero4<false><<<(int)blocks, 256, 0, stream>>>(reinterpret_cast<float4*>(param), reinterpret_cast<float4*>(grad), reinterpret_cast<float4*>(exp_avg),
+                                                         reinterpret_cast<float4*>(exp_avg_sq), n4, lr, beta1, beta2, eps, (float)bc1, (float)sqrt(bc2),
+                                                         inv_grad_scale, skip_flag, live, HalfDst{});
   return cnb_check_launch("adam_zero");
 }

@@ -203,7 +203,7 @@ int forward_chain(const cnb_model* m, const cnb_rays* rays, const Layout& L, flo
                                                     (lv + 1 == lf && user) ? out->pdf_inds : nullptr, st));
       if (rc) return rc;
     } else {
-      STAGE("field_fwd", mixed_wide ? cnb_field_mixed_wide_launches(&m->field, false, false) : (mixed ? 1 : 7), cnb_field_fwd(&m->field, &sm, ws + L.dens[lv], nullptr, ws + L.rgb, ws + L.sem, nullptr,
+      STAGE("field_fwd", mixed_wide ? cnb_field_mixed_wide_launches(&m->field, false, false) : (mixed ? 1 : 7), cnb_field_fwd_half(&m->field, m->field_table_half, &sm, ws + L.dens[lv], nullptr, ws + L.rgb, ws + L.sem, nullptr,
                                                         L.ctx_floats > 0 ? ws + L.ctx : nullptr, training ? 1 : 0, st));
       if (rc) return rc;
     }
@@ -300,7 +300,15 @@ extern "C" int cnb_train_step(const cnb_model* m, const cnb_rays* rays, const cn
     for (int i = 0; i < cfg->num_opt_groups; ++i) {
       const cnb_opt_group& og = cfg->opt_groups[i];
       if (og.chain != chain) continue;
-      if (og.peer_comm != nullptr)  // data parallel over peer memory: the group's whole exchange on this chain's branch
+      const cnb_opt_half& oh = cfg->opt_half[i];
+      if (oh.table_half != nullptr && og.peer_comm != nullptr) {
+        cnb_set_error("train_step: the peer-memory exchange does not refresh fp16 table copies");
+        return CNB_ERR_UNSUPPORTED;
+      }
+      if (oh.table_half != nullptr)  // the group holds a table with an fp16 copy: the update refreshes it from registers
+        STAGE(chain == CNB_CHAIN_FIELD ? "adam_fields" : "adam_proposals", 1, cnb_adam_step_zero_dev_half(og.param, og.grad, og.exp_avg, og.exp_avg_sq, og.n,
+                                                                                                         og.scalars, og.live, oh.table_half, oh.first, oh.count, st));
+      else if (og.peer_comm != nullptr)  // data parallel over peer memory: the group's whole exchange on this chain's branch
         STAGE(chain == CNB_CHAIN_FIELD ? "exchange_fields" : "exchange_proposals", 3, cnb_ddp_exchange_dev(og.peer_comm, og.peer_group, og.exp_avg, og.exp_avg_sq,
                                                                                                           og.grad, og.n, og.scalars, og.peer_flags, og.peer_channel, st));
       else
@@ -317,8 +325,8 @@ extern "C" int cnb_train_step(const cnb_model* m, const cnb_rays* rays, const cn
                                                             m->field.pass_semantic_gradients, losses_out, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, st));
     if (rc) return rc;
     const cnb_samples sm = make_samples(rays, ws + L.eu[lf], Sf);
-    if (rays_grad) STAGE("field_bwd", mixed_wide ? cnb_field_mixed_wide_launches(&m->field, true, true) : (mixed ? 3 : 9), cnb_field_bwd_rays(&m->field, &sm, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, nullptr, ws + L.ctx,
-                                                                        d_origins, d_directions, st));
+    if (rays_grad) STAGE("field_bwd", mixed_wide ? cnb_field_mixed_wide_launches(&m->field, true, true) : (mixed ? 3 : 9), cnb_field_bwd_rays_half(&m->field, m->field_table_half, &sm, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, nullptr,
+                                                                        ws + L.ctx, d_origins, d_directions, st));
     else STAGE("field_bwd", mixed_wide ? cnb_field_mixed_wide_launches(&m->field, true, false) : (mixed ? 2 : 8), cnb_field_bwd(&m->field, &sm, ws + L.d_dens[lf], ws + L.d_rgb, ws + L.d_sem, nullptr, ws + L.ctx, st));
     if (rc) return rc;
     return optimise(CNB_CHAIN_FIELD, st);  // the field gradient is complete: its Adam pass overlaps the proposal chain
@@ -389,6 +397,7 @@ extern "C" int cnb_train_step(const cnb_model* m, const cnb_rays* rays, const cn
     for (int i = 0; i < cfg->num_opt_groups; ++i) {
       const cnb_opt_group& og = cfg->opt_groups[i];
       if (og.chain != CNB_CHAIN_JOIN) continue;
+      CNB_REQUIRE(cfg->opt_half[i].table_half == nullptr, "train_step: the camera-optimizer group holds no hash table");
       STAGE("adam_camera_opt", 1, cnb_adam_step_zero_dev_live(og.param, og.grad, og.exp_avg, og.exp_avg_sq, og.n, og.scalars, og.live, stream));
       if (rc) return rc;
     }

@@ -145,6 +145,7 @@ class FlatGroup:
         dev = uniq[0].device
         self.peer = None
         self.live = None
+        self.half = None   # (fp16 copy, first float, float count) of a hash table in the group whose copy the update refreshes (Trainer)
         if comm is not None:
             from .ddp import PeerGroup
 
@@ -271,7 +272,7 @@ class _GraphedStep:
                     mm = trainer.ddp == "p2p_multimem" and g.peer.has_multicast
                     pinfo = (trainer.comm.struct, g.peer.struct, (L_.P2P_GRADS_ZERO if zero else 0) | (L_.P2P_MULTIMEM if mm else 0), 2 + (i & 1))
                 chain = {"fields": L_.CHAIN_FIELD, "proposal_networks": L_.CHAIN_PROPOSALS, "camera_opt": L_.CHAIN_JOIN}[n]
-                self.opt.append((g.flat, g.grad, g.exp_avg, g.exp_avg_sq, self.opt_dev[i], chain, g.live, pinfo))
+                self.opt.append((g.flat, g.grad, g.exp_avg, g.exp_avg_sq, self.opt_dev[i], chain, g.live, pinfo, g.half))
             self.opt_names = names
             self.inv_world = 1.0 / trainer.world_size
         self.graph = torch.cuda.CUDAGraph()
@@ -417,7 +418,8 @@ class Trainer:
         """``ddp`` (world_size > 1): "nccl" = all-reduce of the flat gradients + local Adam (DDP as the reference does it);
         "p2p" = one reduce-scatter + Adam + all-gather kernel per group over NVLink peer mappings (csrc/ddp_p2p.cu);
         "p2p_multimem" = the same through the NVLS multicast mappings; "auto" = p2p when the symmetric-memory rendezvous works
-        (CUDA, peer access), else nccl.  A GradScaler needs the global inf/NaN verdict before any update: it keeps nccl."""
+        (CUDA, peer access), else nccl.  A GradScaler needs the global inf/NaN verdict before any update: it keeps nccl.  So do fp16 field
+        tables (FruitField table_precision="fp16"): the peer-memory exchange does not refresh their copy, and "p2p*" refuses them."""
         from .pipeline import FusedPipeline
 
         self.model = model
@@ -442,7 +444,11 @@ class Trainer:
         self._camopt_eager = _os.environ.get("CNB_CAMOPT_EAGER", "0") == "1"
         self.check_peers_every = 64       # peer-memory mode: read the barrier time-out flag every N steps (and before checkpoints)
         self.ddp = "nccl"
-        if world_size > 1 and ddp != "nccl" and self.grad_scaler is None and next(model.parameters()).is_cuda:
+        field = getattr(model, "field", None)
+        fp16_tables = getattr(field, "table_precision", "fp32") == "fp16"
+        if fp16_tables and world_size > 1 and ddp in ("p2p", "p2p_multimem"):
+            raise ValueError(f"ddp={ddp!r} does not refresh the fp16 copy of the field table (table_precision='fp16'): use ddp='nccl'")
+        if world_size > 1 and ddp != "nccl" and self.grad_scaler is None and not fp16_tables and next(model.parameters()).is_cuda:
             try:
                 from .ddp import PeerComm
 
@@ -463,8 +469,23 @@ class Trainer:
         if _os.environ.get("CNB_NO_LIVE_MASK", "0") != "1" and next(model.parameters()).is_cuda:
             for g in self.groups.values():
                 g.build_live(model)
+        if fp16_tables:
+            # every update of the fields group also writes the fp16 copy of the field table (from registers: one 8-byte store per float4)
+            g, t = self.groups["fields"], field.mlp_base_grid.hash_table
+            first = (t.data_ptr() - g.flat.data_ptr()) // 4
+            if not 0 <= first <= g.flat.numel() - t.numel():
+                raise RuntimeError("the field hash table is not inside the fields parameter group")
+            g.half = (field.table_half, first, t.numel())
         self.callbacks = model.get_training_callbacks()
         self.opt_step = 0
+
+    def _refresh_table_copy(self) -> None:
+        """fp16 field tables: a write made outside the trainer since the last step (checkpoint load, an in-place copy) is copied into the fp16
+        table before the step reads it; re-homing the parameters into the flat group counts as such a write."""
+        field = getattr(self.model, "field", None)
+        if field is not None and getattr(field, "table_precision", "fp32") == "fp16" and field.table_copy_stale():
+            self.wait_deferred_update()
+            field.refresh_table_copy()
 
     def _run_callbacks(self, where: str, step: int) -> None:
         for cb in self.callbacks:
@@ -525,10 +546,10 @@ class Trainer:
             if spec.kind != "adam":
                 if flag is not None:
                     raise NotImplementedError("RAdam with a GradScaler: the guarded update kernel computes Adam's bias corrections itself")
-                ops.adam_step_scalars(g.flat, g.grad, g.exp_avg, g.exp_avg_sq, step_scalars(spec, lr, self.opt_step, inv), live=g.live)
+                ops.adam_step_scalars(g.flat, g.grad, g.exp_avg, g.exp_avg_sq, step_scalars(spec, lr, self.opt_step, inv), live=g.live, half=g.half)
                 continue
             ops.adam_step(g.flat, g.grad, g.exp_avg, g.exp_avg_sq, lr, self.opt_step, spec.betas[0], spec.betas[1], spec.eps,
-                          inv_grad_scale=inv, zero_grad=True, skip_flag=flag, live=g.live)
+                          inv_grad_scale=inv, zero_grad=True, skip_flag=flag, live=g.live, half=g.half)
         self._grads_clean = True
         if scaler is not None and scaler.update():
             self.opt_step -= 1  # torch: a skipped optimizer.step() does not advance Adam's step count
@@ -595,10 +616,11 @@ class Trainer:
         spec = self.optimizers["fields"]
         with torch.cuda.stream(self._side_stream):
             if spec.kind != "adam":
-                ops.adam_step_scalars(g.flat, g.grad, g.exp_avg, g.exp_avg_sq, step_scalars(spec, exponential_decay_lr(step, spec), self.opt_step), live=g.live)
+                ops.adam_step_scalars(g.flat, g.grad, g.exp_avg, g.exp_avg_sq, step_scalars(spec, exponential_decay_lr(step, spec), self.opt_step), live=g.live,
+                                      half=g.half)
             else:
                 ops.adam_step(g.flat, g.grad, g.exp_avg, g.exp_avg_sq, exponential_decay_lr(step, spec), self.opt_step, spec.betas[0], spec.betas[1],
-                              spec.eps, inv_grad_scale=1.0, zero_grad=True, live=g.live)
+                              spec.eps, inv_grad_scale=1.0, zero_grad=True, live=g.live, half=g.half)
             self._deferred_event.record(self._side_stream)
         self._deferred_pending = True
         self.model._param_fence = self.wait_deferred_update
@@ -642,6 +664,7 @@ class Trainer:
         if not self.model.training:  # nn.Module.train() walks every sub-module: only when the mode actually changes
             self.model.train()
         self._run_callbacks("BEFORE_TRAIN_ITERATION", step)
+        self._refresh_table_copy()
         self.model._params_version = getattr(self.model, "_params_version", 0) + 1  # invalidates the eval path's cached descriptors
         graphed = False
         if not getattr(self, "_grads_clean", False):

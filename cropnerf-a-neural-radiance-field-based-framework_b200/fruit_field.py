@@ -48,6 +48,7 @@ class FruitField(nn.Module):
         spatial_distortion: Optional[nn.Module] = None,
         implementation: str = "b200",
         precision: str = "fp32",
+        table_precision: str = "fp32",
     ) -> None:
         super().__init__()
         if not use_semantics or num_semantic_classes != 1:
@@ -82,6 +83,55 @@ class FruitField(nn.Module):
         self._cache: Optional[tuple] = None
         self._sample_locations: Optional[Tensor] = None
         self._density_before_activation: Optional[Tensor] = None
+        self.table_precision = table_precision
+        if table_precision not in ("fp32", "fp16"):
+            raise ValueError(f"table_precision {table_precision!r}: 'fp32' or 'fp16'")
+        if table_precision == "fp16":
+            if precision != "mixed":
+                raise ValueError("table_precision='fp16' needs precision='mixed': exact fp32 mode evaluates the fp32 table (it is the parity reference)")
+            if self._fused_base_architecture():
+                raise ValueError("table_precision='fp16' is built for fields wider than the fused base-preset kernels (the fruit_nerf_big / _huge "
+                                 "presets): the base preset's 64 MiB table fits the B200's L2, where fp16 rows gather no faster than fp32 rows "
+                                 "(DESIGN.md section 7)")
+            # the fp16 copy the field forward gathers; the fp32 hash_table stays the parameter (optimiser, gradients, checkpoints)
+            self.register_buffer("table_half", torch.zeros(self.mlp_base_grid.hash_table.shape, dtype=torch.float16), persistent=False)
+            self._half_stamp: Optional[tuple] = None
+
+    def _fused_base_architecture(self) -> bool:
+        """The shapes csrc/field_mixed.cu compiles (cnb_field_mixed_supported): the base preset."""
+        dims = lambda m: [m.layers[0].in_features] + [l.out_features for l in m.layers]  # noqa: E731
+        return (self.mlp_base_grid.num_levels <= 16 and dims(self.mlp_base_mlp)[1:] == [64, 16] and dims(self.mlp_semantics) == [15, 64, 64]
+                and dims(self.mlp_head) == [63, 64, 64, 3] and self.appearance_embedding_dim == 32 and self.geo_feat_dim == 15)
+
+    # ------------------------------------------------------------------------------------------------
+    # fp16 tables (table_precision="fp16").  The copy is kept in step by the optimiser (engine.Trainer fuses the refresh into every flat-group
+    # update) and refreshed here whenever the table was written any other way: an in-place torch write (load_state_dict,
+    # hash_table.copy_ under no_grad) bumps the parameter's version counter, re-homing it changes its storage.  A write through
+    # ``hash_table.data`` bumps neither: call refresh_table_copy() after one.
+    def _table_stamp(self) -> tuple:
+        t = self.mlp_base_grid.hash_table
+        return (t._version, t.data_ptr(), t.device, self.table_half.data_ptr())
+
+    def table_copy_stale(self) -> bool:
+        return self.table_precision == "fp16" and self._half_stamp != self._table_stamp()
+
+    def refresh_table_copy(self) -> None:
+        """Rewrite the fp16 copy from the fp32 hash_table (``__float2half_rn`` of every value)."""
+        if self.table_precision != "fp16":
+            return
+        t = self.mlp_base_grid.hash_table
+        if self.table_half.device != t.device:
+            self.table_half = self.table_half.to(t.device)
+        ops.table_to_half(t.detach(), self.table_half)
+        self._half_stamp = self._table_stamp()
+
+    def table_half_current(self) -> Optional[Tensor]:
+        """The fp16 copy the field forward gathers (refreshed first when stale), or None for fp32 tables."""
+        if self.table_precision != "fp16":
+            return None
+        if self.table_copy_stale():
+            self.refresh_table_copy()
+        return self.table_half
 
     # ------------------------------------------------------------------------------------------------
     def kernel_params(self):
@@ -115,6 +165,7 @@ class FruitField(nn.Module):
             "appearance_mode": self._appearance_mode(inference),
             "pass_semantic_gradients": self.pass_semantic_gradients,
             "precision": L.PREC_MIXED if self.precision == "mixed" else L.PREC_FP32,
+            "table_half": self.table_half_current(),
             "training": torch.is_grad_enabled(),
             "want_positions": True,
         }

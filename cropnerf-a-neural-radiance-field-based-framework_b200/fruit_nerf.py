@@ -76,6 +76,9 @@ class FruitNerfModelConfig:
     geo_feat_dim: int = 15
     # B200 selector: "fp32" (exact, 1e-4 parity) or "mixed" (fp16 tensor-core MLPs, 2e-3 parity)
     precision: str = "fp32"
+    # hash-table storage the field forward gathers: "fp32", or "fp16" (a copy the optimiser keeps in step with the fp32 master table; only with
+    # precision="mixed" on fields wider than the fused base-preset kernels, i.e. the big / huge presets -- FruitField raises otherwise)
+    table_precision: str = "fp32"
 
     def setup(self, **kwargs) -> "FruitModel":
         return FruitModel(self, **kwargs)
@@ -236,6 +239,7 @@ class FruitModel(nn.Module):
             num_semantic_classes=1,
             pass_semantic_gradients=cfg.pass_semantic_gradients,
             precision=cfg.precision,
+            table_precision=cfg.table_precision,
         )
         self.camera_optimizer = CameraOptimizer(self.num_train_data, cfg.camera_optimizer_mode)
         self.density_fns: List[Callable] = []

@@ -50,6 +50,7 @@ else:
         hidden_dim_semantics: int = 64
         geo_feat_dim: int = 15
         precision: str = "mixed"   # the reference preset trains with mixed_precision=True (fruit_nerf_config.py:35)
+        table_precision: str = "fp32"   # "fp16": fp16 hash-table gathers for the big / huge presets in mixed precision (FruitField)
 
     class FruitModelB200(Model):
         """nerfstudio ``Model`` whose modules are this package's (``FruitModel.populate_modules``, fruit_nerf.py:87-183).  Every method

@@ -269,8 +269,8 @@ class _FieldFn(torch.autograd.Function):
         geo = torch.empty((N, 1 + cfg["geo_feat_dim"]), device=dev, dtype=torch.float32) if want_geo else None
         pos = torch.empty((N, 3), device=dev, dtype=torch.float32) if cfg.get("want_positions", True) else None
         L.check(
-            lib.cnb_field_fwd(C.byref(f), C.byref(sm), density.data_ptr(), _p(geo), rgb.data_ptr(), sem.data_ptr(), _p(pos),
-                              scratch.data_ptr() if ctx_floats > 0 else None, int(training), L.stream_ptr(dev)),
+            lib.cnb_field_fwd_half(C.byref(f), _p(cfg.get("table_half")), C.byref(sm), density.data_ptr(), _p(geo), rgb.data_ptr(), sem.data_ptr(),
+                                   _p(pos), scratch.data_ptr() if ctx_floats > 0 else None, int(training), L.stream_ptr(dev)),
             "field_fwd",
         )
         ctx.cfg, ctx.layout, ctx.training = cfg, layout, training
@@ -305,8 +305,8 @@ class _FieldFn(torch.autograd.Function):
         d_o = d_d = None
         if ctx.rays_grad:  # row a17: gradient with respect to the rays (camera optimizer)
             d_o, d_d = torch.zeros_like(origins), torch.zeros_like(directions)
-            L.check(L.lib().cnb_field_bwd_rays(C.byref(f), C.byref(sm), _p(dd), _p(dr), _p(ds), _p(dg), scratch_ptr, d_o.data_ptr(), d_d.data_ptr(),
-                                               L.stream_ptr(dev)), "field_bwd_rays")
+            L.check(L.lib().cnb_field_bwd_rays_half(C.byref(f), _p(cfg.get("table_half")), C.byref(sm), _p(dd), _p(dr), _p(ds), _p(dg), scratch_ptr,
+                                                    d_o.data_ptr(), d_d.data_ptr(), L.stream_ptr(dev)), "field_bwd_rays")
         else:
             L.check(L.lib().cnb_field_bwd(C.byref(f), C.byref(sm), _p(dd), _p(dr), _p(ds), _p(dg), scratch_ptr, L.stream_ptr(dev)), "field_bwd")
         # the mean-embedding gradient is not propagated (inference-only mode, fruit_field.py:219-221)
@@ -564,10 +564,29 @@ def pixel_losses(rgb: Tensor, sem: Tensor, image: Tensor, mask: Tensor, sem_weig
 # ---------------------------------------------------------------------------------------------------------
 
 
+def table_to_half(table: Tensor, table_half: Tensor, live: Optional[Tensor] = None, first_unit: int = 0) -> None:
+    """table_half = table.half() (``__float2half_rn``); with ``live`` (a flat group's reachable bitmap, the table at 16-byte unit
+    ``first_unit``) only the units the optimiser updates are written."""
+    dev = _dev(table)
+    if table_half.dtype != torch.float16 or table_half.numel() != table.numel() or not table_half.is_contiguous() or not table.is_contiguous():
+        raise ValueError("table_to_half: table_half must be a contiguous float16 tensor with the table's size")
+    L.check(L.lib().cnb_table_to_half(table.data_ptr(), table.numel(), _p(live), int(first_unit), table_half.data_ptr(), L.stream_ptr(dev)), "table_to_half")
+
+
 def adam_step(param: Tensor, grad: Tensor, exp_avg: Tensor, exp_avg_sq: Tensor, lr: float, step: int, beta1: float = 0.9, beta2: float = 0.999,
               eps: float = 1e-15, inv_grad_scale: float = 1.0, zero_grad: bool = False, skip_flag: Optional[Tensor] = None,
-              live: Optional[Tensor] = None) -> None:
+              live: Optional[Tensor] = None, half: Optional[tuple] = None) -> None:
+    """``half`` = (fp16 table copy, first float, float count) of a hash table inside the group (engine.FlatGroup.half): the update also stores
+    every table value it writes into the copy."""
     dev = _dev(param)
+    if half is not None:
+        if not zero_grad:
+            raise ValueError("adam_step: the fp16 table refresh is fused into the update + gradient-clear pass (zero_grad=True)")
+        tab, first, count = half
+        L.check(L.lib().cnb_adam_step_zero_half(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), param.numel(), lr, beta1,
+                                                beta2, eps, int(step), inv_grad_scale, _p(skip_flag), _p(live), tab.data_ptr(), int(first), int(count),
+                                                L.stream_ptr(dev)), "adam_step_half")
+        return
     if live is not None and zero_grad and skip_flag is None:  # skip the units no hash-grid corner can reach (bit-identical, see reachable_bitmap)
         L.check(L.lib().cnb_adam_step_zero_live(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), param.numel(), lr, beta1,
                                                 beta2, eps, int(step), inv_grad_scale, live.data_ptr(), L.stream_ptr(dev)), "adam_step_live")
@@ -584,12 +603,17 @@ def adam_step(param: Tensor, grad: Tensor, exp_avg: Tensor, exp_avg_sq: Tensor, 
     )
 
 
-def adam_step_scalars(param: Tensor, grad: Tensor, exp_avg: Tensor, exp_avg_sq: Tensor, scalars, live: Optional[Tensor] = None) -> None:
+def adam_step_scalars(param: Tensor, grad: Tensor, exp_avg: Tensor, exp_avg_sq: Tensor, scalars, live: Optional[Tensor] = None,
+                      half: Optional[tuple] = None) -> None:
     """The flat-group update + gradient clear with the step's seven scalars given explicitly (engine.step_scalars: Adam or RAdam):
     ``p -= (s0 / s4) * m / (sqrt(v) / s5 + s3)``.  The scalars travel as one 28-byte device tensor (cnb_adam_step_zero_dev[_live])."""
     dev = _dev(param)
     sc = torch.tensor([float(x) for x in scalars] + [0.0], dtype=torch.float32).to(dev, non_blocking=False)
-    if live is not None:
+    if half is not None:  # (fp16 table copy, first float, float count): see adam_step
+        tab, first, count = half
+        L.check(L.lib().cnb_adam_step_zero_dev_half(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), param.numel(),
+                                                    sc.data_ptr(), _p(live), tab.data_ptr(), int(first), int(count), L.stream_ptr(dev)), "adam_step_dev_half")
+    elif live is not None:
         L.check(L.lib().cnb_adam_step_zero_dev_live(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), param.numel(),
                                                     sc.data_ptr(), live.data_ptr(), L.stream_ptr(dev)), "adam_step_dev_live")
     else:

@@ -61,6 +61,7 @@ class FusedPipeline:
         load_state_dict -- ``model._params_version`` --, mode switches, background colour)."""
         m = self.model
         if not with_grads:
+            m.field.table_half_current()  # a stale fp16 table copy is refreshed in place: the cached descriptor's pointer stays valid
             tab = m.field.mlp_base_grid.hash_table
             key = (str(dev), training, ray_gradients, m.field.test_mode, getattr(m, "_params_version", 0), tab.data_ptr(), m.field.spatial_distortion is None,
                    str(m.renderer_rgb.background_color), getattr(m.config, "precision", "fp32"), tuple(int(v) for v in m.proposal_sampler.num_proposal_samples_per_ray),
@@ -92,6 +93,8 @@ class FusedPipeline:
         keep.append(k)
         ms = L.Model()
         ms.field = fs
+        if fcfg["table_half"] is not None:
+            ms.field_table_half = fcfg["table_half"].data_ptr()
         s = m.proposal_sampler
         n = s.num_proposal_network_iterations
         for i in range(n):
@@ -279,6 +282,9 @@ class FusedPipeline:
                 og.live = live_.data_ptr() if live_ is not None else None
                 og.param, og.grad, og.exp_avg, og.exp_avg_sq = p_.data_ptr(), g_.data_ptr(), m_.data_ptr(), v_.data_ptr()
                 og.n, og.scalars, og.chain = p_.numel(), sc_.data_ptr(), int(chain)
+                if len(entry) > 8 and entry[8] is not None:  # the group's fp16 table copy (engine.FlatGroup.half), refreshed by its update
+                    tab_, first_, count_ = entry[8]
+                    cfg.opt_half[i].table_half, cfg.opt_half[i].first, cfg.opt_half[i].count = tab_.data_ptr(), int(first_), int(count_)
                 if len(entry) > 7 and entry[7] is not None:
                     # peer-memory data parallelism: this group's whole exchange runs inside the step (cnb_opt_group.peer_*); the structs are
                     # read at enqueue time, the entry keeps them alive

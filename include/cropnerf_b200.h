@@ -133,6 +133,14 @@ int cnb_device_count(void);
 int cnb_hashgrid_fwd(const cnb_grid* g, const float* positions, int64_t n, float* out, int32_t* indices, cnb_stream_t stream);
 /* accumulates g->d_table from d_out [n, 2*L] */
 int cnb_hashgrid_bwd(const cnb_grid* g, const float* positions, const float* d_out, int64_t n, cnb_stream_t stream);
+/* fp16 table rows (fruit_nerf_big / _huge with table_precision="fp16"): table_half [num_levels * 2^log2_hashmap_size] __half2 (8-byte aligned)
+ * is gathered instead of g->table; each corner is widened to fp32 and blended as in cnb_hashgrid_fwd, so the result equals cnb_hashgrid_fwd on a
+ * table holding table_half's values.  table_half NULL = cnb_hashgrid_fwd. */
+int cnb_hashgrid_fwd_half(const cnb_grid* g, const void* table_half, const float* positions, int64_t n, float* out, int32_t* indices,
+                          cnb_stream_t stream);
+/* table_half[i] = __float2half_rn(table[i]) for n floats (n % 4 == 0; table 16-byte, table_half 8-byte aligned).  live (optional) = a flat
+ * group's bitmap (cnb_hashgrid_mark_reachable) with the table at unit first_unit: only units whose bit is set are written. */
+int cnb_table_to_half(const float* table, int64_t n, const uint32_t* live, int64_t first_unit, void* table_half, cnb_stream_t stream);
 
 /* ---- a3/a4: MLP / FieldHead (nerfstudio mlp.py, field_heads.py; fruit_field.py:133-141,146-154,159-167;
  *      SemanticFieldHead components/field_heads.py:29-40, used fruit_field.py:155-157,207,269) ---------------------------------- */
@@ -184,6 +192,11 @@ int cnb_field_fwd(const cnb_field* f, const cnb_samples* s, float* density, floa
 /* d_geo (optional) [N,1+geo] external gradient on the geo embedding; accumulates all parameter gradients */
 int cnb_field_bwd(const cnb_field* f, const cnb_samples* s, const float* d_density, const float* d_rgb, const float* d_sem,
                   const float* d_geo, float* ctx, cnb_stream_t stream);
+/* cnb_field_fwd gathering the fp16 copy of f->grid.table (see cnb_hashgrid_fwd_half); table_half NULL = cnb_field_fwd.  Compiled for
+ * precision CNB_PREC_MIXED on the layer-by-layer path only (MLPs outside the fused base kernels); elsewhere CNB_ERR_UNSUPPORTED.  The backward
+ * (cnb_field_bwd) reads no table; cnb_field_bwd_rays_half differentiates the same fp16 rows. */
+int cnb_field_fwd_half(const cnb_field* f, const void* table_half, const cnb_samples* s, float* density, float* geo, float* rgb, float* sem,
+                       float* positions_out, float* ctx, int32_t training, cnb_stream_t stream);
 
 /* ---- a17: gradient with respect to the rays (camera optimizer, fruit_nerf.py:114-116,547,614) ---------------------- */
 /* d_feat [N, 2L] = gradient reaching a grid's encoded features; accumulates d_origins / d_directions [R,3]:
@@ -196,6 +209,11 @@ int cnb_density_field_bwd_rays(const cnb_density_field* f, const cnb_samples* s,
 /* cnb_field_bwd + ray gradients (the SH direction encoding carries no gradient, as in nerfstudio's torch SHEncoding) */
 int cnb_field_bwd_rays(const cnb_field* f, const cnb_samples* s, const float* d_density, const float* d_rgb, const float* d_sem,
                        const float* d_geo, float* ctx, float* d_origins, float* d_directions, cnb_stream_t stream);
+/* the two with the fp16 table copy the forward gathered (cnb_field_fwd_half) */
+int cnb_position_grad_rays_half(const cnb_grid* g, const void* table_half, const cnb_warp* warp, const cnb_samples* s, const float* d_feat,
+                                float* d_origins, float* d_directions, cnb_stream_t stream);
+int cnb_field_bwd_rays_half(const cnb_field* f, const void* table_half, const cnb_samples* s, const float* d_density, const float* d_rgb,
+                            const float* d_sem, const float* d_geo, float* ctx, float* d_origins, float* d_directions, cnb_stream_t stream);
 
 /* ---- a8/a9: samplers (nerfstudio ray_samplers.py; components/ray_samplers.py:54-104) ----------------------- */
 /* SpacedSampler: lin_bins = torch.linspace(0,1,S+1) supplied by the host (bit-exact u); t_rand NULL (eval) or
@@ -382,6 +400,7 @@ typedef struct cnb_model {
   int32_t bg_mode;                 /* CNB_BG_* (renderer_rgb background_color / override context) */
   float bg_color[3];
   int32_t ray_gradients;           /* training workspace also holds the scratch for cnb_train_cfg.d_origins / d_directions */
+  const void* field_table_half;    /* fp16 copy of field.grid.table (cnb_field_fwd_half), or NULL = the fp32 table */
 } cnb_model;
 
 /* per-ray outputs, each optional (NULL = not wanted) */
@@ -425,6 +444,12 @@ typedef struct cnb_opt_group {
   int32_t peer_channel;      /* barrier channel 0..3 reserved for this stage */
 } cnb_opt_group;
 
+/* the fp16 copy of a hash table inside an optimiser group (cnb_adam_step_zero_dev_half): table_half = NULL for none */
+typedef struct cnb_opt_half {
+  void* table_half;
+  int64_t first, count;      /* float range of the table inside the group, multiples of 4 */
+} cnb_opt_half;
+
 typedef struct cnb_train_cfg {
   const float* image;        /* [R,3] target colours */
   const float* fruit_mask;   /* [R] 0/1 */
@@ -455,6 +480,7 @@ typedef struct cnb_train_cfg {
   int32_t num_cameras;
   float trans_l2_penalty, rot_l2_penalty;
   int32_t _pad_camopt;
+  cnb_opt_half opt_half[CNB_MAX_OPT_GROUPS];  /* per opt_groups entry; refused with peer-memory groups and the camera-optimizer group */
 } cnb_train_cfg;
 
 /* forward + losses + backward of one batch; parameter gradients are ACCUMULATED into the d_* pointers of `m`;
@@ -495,6 +521,16 @@ int cnb_adam_step_zero_dev_live(float* param, float* grad, float* exp_avg, float
 int cnb_grad_check_finite(const float* grad, int64_t n, int32_t* found_inf, cnb_stream_t stream);
 int cnb_adam_step_zero_guarded(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1, float beta2,
                                float eps, int32_t step, float inv_grad_scale, const int32_t* skip_flag, cnb_stream_t stream);
+
+/* The flat-group updates of a group holding a hash table with an fp16 copy (cnb_table_to_half): the table occupies floats
+ * [half_first, half_first + half_count) of the group (multiples of 4); every float4 of it the update writes is also stored, rounded to fp16, into
+ * table_half -- from registers, without a second pass over the table.  Units left unchanged (live bit 0, a skipped step) keep their copy.
+ * cnb_adam_step_zero_half = cnb_adam_step_zero / _live / _guarded (skip_flag, live optional); cnb_adam_step_zero_dev_half = _dev / _dev_live. */
+int cnb_adam_step_zero_half(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1, float beta2, float eps,
+                            int32_t step, float inv_grad_scale, const int32_t* skip_flag, const uint32_t* live, void* table_half, int64_t half_first,
+                            int64_t half_count, cnb_stream_t stream);
+int cnb_adam_step_zero_dev_half(float* param, float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, const float* scalars, const uint32_t* live,
+                                void* table_half, int64_t half_first, int64_t half_count, cnb_stream_t stream);
 
 /* ---- (e) data-parallel optimiser step over NVLink / NVSwitch peer memory: gradient reduce-scatter + Adam + parameter all-gather in ONE
  * kernel (replaces DDP's all-reduce, fruit_pipeline.py:119-121, followed by torch.optim.Adam, fruit_nerf_config.py:45-60).
